@@ -2,7 +2,7 @@
 """bench.py -- the driver's benchmark contract for nvbio_b200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--genome-mbp 3000] [--reads 1000000] [--workload seed_extend|fm_match|banded_gotoh]
+                    [--genome-mbp 3000] [--reads 1000000] [--workload seed_extend|fm_match|banded_gotoh] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[2] "nvBowtie seed-and-extend: 1M x 150bp single-end, 20bp seeds,
 band=31, synthetic 3Gbp index" -- the configuration the headline metric (Mreads/s, 150 bp, seed+extend) is
@@ -40,7 +40,9 @@ SEED_LEN, SEED_INTERVAL, BAND, READ_LEN = 20, 10, 31, 150
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline seed+extend measurement and of its host-to-host (e2e) leg; the secondary measurements "
+                         "keep their own sizes (paired end: the --c5-total-pairs job; reference-format fm_match and other_configs: best of 5; CPU baseline: one step)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="seed_extend", choices=["seed_extend", "fm_match", "banded_gotoh"])
@@ -59,7 +61,30 @@ def parse():
     ap.add_argument("--pairs", type=int, default=500_000, help="read pairs per GPU per step of the paired-end (C5-shaped) measurement; 0 = skip")
     ap.add_argument("--c5-total-pairs", type=int, default=100_000_000,
                     help="total pairs of the paired-end job (BASELINE configs[4]: 100M), processed as ceil(total / (gpus x pairs)) steps per GPU")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy: per-read best score and position, and the hit "
+                         "counts; the inputs are the same from run to run, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of this project's timed path: not with --impl reference")
+    return args
+
+
+DUMP_MAX_READS = 2_000_000      # 3 float64 arrays of at most 2M entries: 48 MB
+
+
+def dump_outputs(out_dir, ws):
+    """the per-read results of the timed seed+extend step (float64: exact for int32 scores and uint32 positions); above DUMP_MAX_READS reads
+    a fixed, seeded sample of them, identified by read_index"""
+    n = ws.best_score.numel()
+    sel = np.arange(n) if n <= DUMP_MAX_READS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_READS, replace=False))
+    out = {"read_index": sel,
+           "best_score": ws.best_score.cpu().numpy()[sel],
+           "best_pos": ws.best_pos.cpu().numpy().view(np.uint32)[sel],
+           "n_hits": ws.n_hits.cpu().numpy()}          # kept, found, distinct alignment jobs
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -653,8 +678,8 @@ def e2e_single(args, nb, fmi, genome, params, batches, n_reads, wpr, hit_capacit
         last["score"] = sc.clone()
         return chk
     # the timed region starts with an empty pipeline and ends when the last result has been read on the host (fill and drain
-    # included); at least 60 batches, so that the one-off fill / drain (about one and a half batches) does not dominate a short run
-    k_steps = max(args.steps, 60)
+    # included: about one and a half batches, so a run of few steps understates the steady rate)
+    k_steps = args.steps
     run(max(args.warmup, depth))
     barrier(world)
     t0 = time.perf_counter()
@@ -714,6 +739,8 @@ def run_ours(args):
         kept, hits, jobs = [int(v) for v in ws.n_hits.cpu()]
         if kept != hits:
             raise SystemExit("bench: hit capacity %d exceeded (%d hits): results would be truncated" % (hit_capacity, hits))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ws)             # before the untimed steps below overwrite the workspace
     barrier(world)
     # a K-step region of a few ms per step can end before nvidia-smi has sampled it: keep the same load running
     # (untimed) until the sampler holds a handful of in-load samples
@@ -783,7 +810,7 @@ def run_ours(args):
         "e2e": {"value": e2e_value, "unit": "Mreads/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "ms_per_step": e2e_ms,
                 "api": "C ABI nvb_pipeline_submit / nvb_pipeline_wait via nvbio_b200.StreamingSeedExtend (pinned host in/out, %d batches in flight: copy-in, "
                        "compute and copy-out streams; wall clock from an empty pipeline to the last result read on the host)" % args.depth,
-                "steps": max(args.steps, 60), "depth": args.depth, "compute_streams": int(os.environ.get("NVB_PIPELINE_COMPUTE_STREAMS", "1")), "sweep": e2e_alt},
+                "steps": args.steps, "depth": args.depth, "compute_streams": int(os.environ.get("NVB_PIPELINE_COMPUTE_STREAMS", "1")), "sweep": e2e_alt},
         # own kernels per step on the per-read path (the cub scan not counted): strings, seed match (+ its second pass when a k-mer table and
         # the full SA are present), count, read jobs, (shortcut check, scatter: LOCAL with a constant scheme), DP pair kernel, DP generic
         # kernel, init, reduce, finalize

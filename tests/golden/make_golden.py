@@ -8,7 +8,8 @@ The fixtures pin (a) the two banded-Gotoh problems asserted by the reference's o
 (nvbio-test/alignment_test.cu:761-825), (b) seeded random banded problems for every BAND/TYPE the
 reference instantiates, incl. text symbols > 3 and ragged lengths, (c) a small FM-index
 (SA, BWT, occ, SSA, match ranges, locate results) incl. a repetitive text, (d) full-matrix Gotoh scores, sinks and
-tracebacks (gotoh_full.npz; `--only-full` regenerates just that file).
+tracebacks (gotoh_full.npz; `--only-full` regenerates just that file), (e) the reference tree's source files and their line counts
+(reference_files.json, which the documentation's citations are checked against; `--only-files DIR` writes it from the tree at DIR).
 """
 import os
 import sys
@@ -252,7 +253,25 @@ def make_nvbwt_files():
     np.savez_compressed(os.path.join(OUT, "nvbwt_files.npz"), **out)
 
 
+CITED_SUFFIXES = (".h", ".cu", ".cpp", ".cuh", ".cmake", ".md", ".txt")
+
+
+def make_reference_files(tree):
+    import json
+    n_lines = {}
+    for dp, _, files in os.walk(tree):
+        for f in files:
+            if f.endswith(CITED_SUFFIXES):
+                p = os.path.join(dp, f)
+                with open(p, errors="ignore") as fh:
+                    n_lines[os.path.relpath(p, tree)] = sum(1 for _ in fh)
+    with open(os.path.join(OUT, "reference_files.json"), "w") as fh:
+        json.dump(n_lines, fh, indent=0, sort_keys=True)
+
+
 def main():
+    if "--only-files" in sys.argv:
+        make_reference_files(sys.argv[sys.argv.index("--only-files") + 1]); print("wrote reference_files.json"); return
     if "--only-nvbwt" in sys.argv:
         make_nvbwt_files(); print("wrote nvbwt_files.npz"); return
     assert orc.Ref.available(), "build oracle/_ref first: make -C oracle"

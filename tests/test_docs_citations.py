@@ -1,11 +1,12 @@
-"""CPU, dev container only (skipped where /root/reference is absent): every `path:line[-line]` citation of the reference in the
-C ABI header, the C++ mirror, DESIGN.md and INTEGRATION.md names a file that exists in the reference tree and a line range inside it."""
+"""CPU: every `path:line[-line]` citation of the reference in the C ABI header, the C++ mirror, DESIGN.md and INTEGRATION.md names a
+file that exists in the reference tree and a line range inside it.  The tree's source files and their line counts are committed
+(tests/golden/reference_files.json, written by tests/golden/make_golden.py --only-files)."""
+import json
 import os
 import re
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+FILES = os.path.join(ROOT, "tests", "golden", "reference_files.json")
 DOCS = ["include/nvbio_b200.h", "DESIGN.md", "INTEGRATION.md", "oracle/nvb_oracle.c", "oracle/ref_shim.cpp",
         "oracle/ref_cuda_bench.cu", "oracle/orc.py", "oracle/cpu_pipeline.py",
         "nvbio_b200/csrc/common.cuh", "nvbio_b200/csrc/fm_core.cuh", "nvbio_b200/csrc/fm_kernels.cu", "nvbio_b200/csrc/gotoh_core.cuh",
@@ -15,18 +16,12 @@ DOCS = ["include/nvbio_b200.h", "DESIGN.md", "INTEGRATION.md", "oracle/nvb_oracl
 CITE = re.compile(r"([A-Za-z0-9_\-./]+\.(?:h|cu|cpp|cuh|cmake|md|txt)):(\d+)(?:-(\d+))?")
 
 
-def _index():
-    idx = {}
-    for dp, _, files in os.walk(REF):
-        for f in files:
-            idx.setdefault(f, []).append(os.path.join(dp, f))
-    return idx
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
 def test_reference_citations_resolve():
-    idx = _index()
-    n_lines = {}
+    with open(FILES) as f:
+        n_lines = json.load(f)                                  # path in the reference tree -> number of lines
+    idx = {}
+    for p in n_lines:
+        idx.setdefault(os.path.basename(p), []).append(p)
     bad, checked = [], 0
     for doc in DOCS:
         text = open(os.path.join(ROOT, doc), errors="ignore").read()
@@ -40,8 +35,6 @@ def test_reference_citations_resolve():
             cands = [p for p in idx[base] if p.endswith(path)] or idx[base]
             ok = False
             for p in cands:
-                if p not in n_lines:
-                    n_lines[p] = sum(1 for _ in open(p, errors="ignore"))
                 if lo <= hi <= n_lines[p]:
                     ok = True
             checked += 1

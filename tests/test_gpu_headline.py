@@ -6,7 +6,8 @@
     sampled adjacent-suffix order, BWT == text[SA-1], occ counters vs the BWT blocks, L2 == symbol counts,
     text[locate(match(p)) ..] == p;
   * seed + extend on bench.py's own CPU-leg reads: best score per read, every per-hit score / sink and the hit count equal
-    the reference's own templates (oracle/_ref, OpenMP) run over the SAME index, through both pipeline paths."""
+    the reference's own templates (oracle/_ref, OpenMP) run over the SAME index, through both pipeline paths (their outputs'
+    digests are committed, tests/reference_digests.py)."""
 import os
 
 import numpy as np
@@ -19,6 +20,8 @@ from nvbio_b200.strings import PackedStringSet
 from oracle import orc
 from oracle.cpu_pipeline import cpu_seed_extend, gather_2bit
 from tests.gpu_util import require_gpu, host_u32
+from tests.reference_digests import Reference
+from tests.test_gpu_fullsize import live_reference
 
 pytestmark = pytest.mark.gpu
 
@@ -141,20 +144,20 @@ def _unpack_rows(words, L):
     return ((words[:, i >> 4] >> sh) & 3).astype(np.uint8)
 
 
-def test_headline_seed_extend_equals_reference(H):
+def test_headline_seed_extend_equals_reference(H, request):
     """bench.py's CPU-leg read sample (20,000 x 150 bp, 1% substitutions, 0.1% indels, both strands) over the headline index:
     hit count, every per-hit (score, sink) in the reference's slot order and the best score per read == the reference's own
     templates (nvbio::match -> locate -> aln::banded_alignment_score<31> -> max) over the same index in the reference's format"""
-    if not orc.Ref.available():
-        pytest.skip("oracle/_ref/libnvbio_ref.so not present")
-    R = orc.Ref(); R.set_num_threads(len(os.sched_getaffinity(0)))
+    R = Reference(request, live_reference)
     fmi, genome, gwh = H["fmi"], H["genome"], H["gwh"]
-    idx = orc._Index(n=N, primary=fmi.primary, bwt_occ=host_u32(fmi.bwt_occ), ssa=host_u32(fmi.ssa[::16].contiguous()), L2=np.array(fmi.L2, np.uint32))
     n_reads = 20_000
     rw, pos, strand = synth.sample_reads(genome, N, n_reads, READ_LEN, sub_rate=0.01, indel_rate=0.001,
                                          seed=synth.SEED_QUERIES + 7919 * 1000, mut_seed=synth.SEED_MUT + 104729 * 1000)
     rw = rw.contiguous()
-    want = cpu_seed_extend(R, idx, gwh, _unpack_rows(host_u32(rw), READ_LEN), SEED_LEN, SEED_INTERVAL, BAND, 1, SCHEME, True, 100)
+    want = None
+    if R.live:
+        idx = orc._Index(n=N, primary=fmi.primary, bwt_occ=host_u32(fmi.bwt_occ), ssa=host_u32(fmi.ssa[::16].contiguous()), L2=np.array(fmi.L2, np.uint32))
+        want = cpu_seed_extend(R.live, idx, gwh, _unpack_rows(host_u32(rw), READ_LEN), SEED_LEN, SEED_INTERVAL, BAND, 1, SCHEME, True, 100)
     rs = PackedStringSet.fixed(rw.reshape(-1), n_reads, READ_LEN, stride=rw.shape[1] * 16)
     params = nb.SeedExtendParams(seed_len=SEED_LEN, seed_interval=SEED_INTERVAL, band_len=BAND, type=aln.LOCAL, both_strands=True,
                                  max_seed_hits=100, dedup_jobs=True, scheme=aln.SimpleGotohScheme(*SCHEME))
@@ -162,14 +165,14 @@ def test_headline_seed_extend_equals_reference(H):
     ws = nb.seed_extend(fmi, genome, rs, params, hit_capacity=24 * n_reads)
     torch.cuda.synchronize()
     kept, total, jobs = [int(v) for v in ws.n_hits.cpu()]
-    assert kept == total == want["n_hits"] and 0 < jobs <= total
-    assert np.array_equal(ws.best_score.cpu().numpy().astype(np.int64), want["best_score"])
-    assert (want["best_score"] > READ_LEN).mean() > 0.99
+    assert kept == total and 0 < jobs <= total
+    best = ws.best_score.cpu().numpy().astype(np.int64)
+    R.same([total, best], lambda: [want["n_hits"], want["best_score"]])
+    assert (best > READ_LEN).mean() > 0.99
     # the per-hit path: every hit's score in the reference's slot order
     ws2 = nb.seed_extend(fmi, genome, rs, params, hit_capacity=24 * n_reads, keep_hits=True)
     torch.cuda.synchronize()
     assert [int(v) for v in ws2.n_hits.cpu()][:2] == [total, total]
-    assert np.array_equal(ws2.hit_score[:total].cpu().numpy(), want["hit_score"])
-    assert np.array_equal(ws2.hit_read[:total].cpu().numpy() // 2, want["hit_read"])
-    assert np.array_equal(ws2.best_score.cpu().numpy().astype(np.int64), want["best_score"])
+    R.same([ws2.hit_score[:total].cpu().numpy(), ws2.hit_read[:total].cpu().numpy() // 2], lambda: [want["hit_score"], want["hit_read"]])
+    assert np.array_equal(ws2.best_score.cpu().numpy().astype(np.int64), best)
     assert np.array_equal(ws2.best_pos.cpu().numpy(), ws.best_pos.cpu().numpy())

@@ -515,9 +515,10 @@ void nvb_pipeline_traffic(const nvb_pipeline* p, size_t* h2d_bytes, size_t* d2h_
 void nvb_pipeline_destroy(nvb_pipeline* p);
 
 /* Profiling aid (the reference wraps every stage in cuda::Timer, nvBowtie/bowtie2/cuda/aligner_best_approx.h:
- * 219-241): device time in ms of the seven stages of the most recent nvb_seed_extend call -- [fw,rc] strings,
- * seed match (FM-index), hit slots, locate + windows, job de-duplication, banded extension, best-per-read.
- * Synchronises on the call's last event. */
+ * 219-241): device time in ms of the seven stages of the most recent direct nvb_seed_extend, nvb_seed_extend_traceback
+ * or nvb_seed_extend_paired call on the current device -- [fw,rc] strings, seed match (FM-index), hit slots, locate +
+ * windows, job de-duplication, banded extension, best-per-read.  nvb_pipeline batches record no stages (see
+ * nvb_pipeline_result.device_ms).  Synchronises on the call's last event. */
 int nvb_seed_extend_stage_ms(float ms[7]);
 
 #ifdef __cplusplus

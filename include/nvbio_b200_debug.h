@@ -24,7 +24,8 @@ void nvb_debug_traceback_fast(int on);
    copies of the text windows) would cost in resident CTAs per SM */
 void nvb_debug_pair_extra_smem(int bytes);
 
-/* seed + extend composition: 0 = automatic (the per-read path when no per-hit output is requested), 1 = always the per-hit path */
+/* seed + extend composition: 0 = automatic (the per-read path when no per-hit output is requested), 1 = always the per-hit path.
+   This and the two switches below are process-wide; a call reads each of them once */
 void nvb_debug_pipeline_path(int path);
 
 /* seed-match stage of the per-read path with a k-mer table: 1 (default) = seeds on k-mers with three or more occurrences are finished

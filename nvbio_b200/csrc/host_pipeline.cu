@@ -6,7 +6,7 @@
 // slot's own compute stream and a copy-out stream, chained by events; nothing blocks the host until wait().  Consecutive
 // batches use different compute streams, so their kernels may share the SMs (the seed search leaves the integer pipes
 // half idle, the extension leaves DRAM idle).
-#include "common.cuh"
+#include "pipeline_core.cuh"
 #include <cstdlib>
 #include <new>
 #include <vector>
@@ -57,20 +57,24 @@ static nvb_string_set reads_view(const nvb_pipeline* p, const uint32_t* d_words)
     return r;
 }
 
+// batches of one device may run at once: they record no stage events (the slot's ev_start / ev_done time the batch)
 static int run_batch(nvb_pipeline* p, nvb_pipeline::Slot& s, size_t* temp_bytes, void* d_temp)
 {
     const nvb_string_set rs = reads_view(p, s.d_in ? s.d_in : (const uint32_t*)16);
     char* o = s.d_out;
     if (!p->paired)
-        return nvb_seed_extend(&p->fmi, p->d_genome, &rs, p->n_reads, &p->params, p->hit_capacity,
-                               o ? (int32_t*)(o + p->o_score) : (int32_t*)16, o ? (uint32_t*)(o + p->o_pos) : (uint32_t*)16,
-                               o ? (uint32_t*)(o + p->o_nhits) : nullptr, nullptr, nullptr, nullptr, nullptr, d_temp, temp_bytes, s.compute);
+        return seed_extend_impl(&p->fmi, p->d_genome, &rs, p->n_reads, &p->params, p->hit_capacity,
+                                o ? (int32_t*)(o + p->o_score) : (int32_t*)16, o ? (uint32_t*)(o + p->o_pos) : (uint32_t*)16,
+                                o ? (uint32_t*)(o + p->o_nhits) : nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                d_temp, temp_bytes, s.compute, false);
     nvb_pair_out po;
     po.d_pair_score = (int32_t*)(o + p->o_pscore); po.d_pair_flags = (uint32_t*)(o + p->o_pflags);
     po.d_mate_score = (int32_t*)(o + p->o_mscore); po.d_mate_pos = (uint32_t*)(o + p->o_mpos); po.d_mate_strand = (uint8_t*)(o + p->o_mstrand);
     po.d_n_rescue = (uint32_t*)(o + p->o_nrescue);
-    return nvb_seed_extend_paired(&p->fmi, p->d_genome, &rs, p->n_reads / 2u, &p->params, p->hit_capacity, &p->pair, &po,
-                                  (uint32_t*)(o + p->o_nhits), d_temp, temp_bytes, s.compute);
+    // as in nvb_seed_extend_paired: the single-end stage writes the per-read bests into the mate arrays
+    return seed_extend_impl(&p->fmi, p->d_genome, &rs, p->n_reads, &p->params, p->hit_capacity, po.d_mate_score, po.d_mate_pos,
+                            (uint32_t*)(o + p->o_nhits), nullptr, nullptr, nullptr, nullptr, nullptr, &p->pair, &po,
+                            d_temp, temp_bytes, s.compute, false);
 }
 
 extern "C" void nvb_pipeline_destroy(nvb_pipeline* p)

@@ -13,6 +13,7 @@
 #include "gotoh_core.cuh"
 #include "pipeline_core.cuh"
 #include <cub/device/device_scan.cuh>
+#include <atomic>
 #include <mutex>
 
 namespace nvb {
@@ -161,10 +162,7 @@ pipe_seed_match_kernel(const FmIndex f, const PipeGeom g, const uint32_t* __rest
                     fm_match_one<BITS, true>(f, words, s * g.stride + pos, g.seed_len, 0u, x, y);
             }
             ranges[q] = make_uint2(x, y);
-            if (!deferred) {
-                const uint32_t sz = (y == 0xFFFFFFFFu) ? 1u : ((x <= y) ? (y - x + 1u) : 0u);
-                sizes[q] = sz < g.max_seed_hits ? sz : g.max_seed_hits;
-            }
+            if (!deferred) sizes[q] = seed_range_size(make_uint2(x, y), g.max_seed_hits);
         }
         if (DEFER) {
             // one atomic per warp, spread over SEED_TODO_LISTS counters, each in its own 128-byte line.  Measured (C3, 0.9 M atomics per
@@ -201,8 +199,7 @@ pipe_seed_match_wide_kernel(const FmIndex f, const PipeGeom g, const uint32_t* _
         uint32_t x = r.x, y = r.y;
         if (fm_match_locate_one<BITS, true, FM_RESUME>(f, genome, words, s * g.stride + k * g.seed_interval, g.seed_len, x, y) == FM_EMPTY) { x = 1; y = 0; }
         ranges[q] = make_uint2(x, y);
-        const uint32_t sz = (y == 0xFFFFFFFFu) ? 1u : ((x <= y) ? (y - x + 1u) : 0u);
-        sizes[q] = sz < g.max_seed_hits ? sz : g.max_seed_hits;
+        sizes[q] = seed_range_size(make_uint2(x, y), g.max_seed_hits);
     }
 }
 
@@ -244,14 +241,10 @@ pipe_expand_hits_kernel(const FmIndex f, const PipeGeom g, const uint2* __restri
     for (uint32_t j = 0; j < sz; ++j) {
         const uint32_t h = base + j;
         if (h >= kept) break;                                                      // beyond the caller's capacity
-        const uint32_t pos = fm_locate_one(f, x + j);
-        const uint32_t diag = pos > seed_begin ? pos - seed_begin : 0u;               // text position of read offset 0
-        const uint32_t gb = diag > g.band / 2u ? diag - g.band / 2u : 0u;             // fmmap.cu:198-199
-        const uint64_t ge64 = (uint64_t)gb + len + g.band;
-        const uint32_t ge = ge64 < g.genome_len ? (uint32_t)ge64 : g.genome_len;
+        const uint2 w = hit_window(fm_locate_one(f, x + j), seed_begin, len, g.band, g.genome_len);
         hit_string[h] = s;
         p_off[h] = s * g.stride; p_len[h] = len;
-        t_off[h] = gb;           t_len[h] = ge - gb;
+        t_off[h] = w.x;          t_len[h] = w.y - w.x;
     }
 }
 
@@ -289,20 +282,16 @@ pipe_read_jobs_kernel(const FmIndex f, const PipeGeom g, const uint2* __restrict
             for (uint32_t k = 0; k < g.seeds_per_string; ++k) {
                 const uint32_t q = s * g.seeds_per_string + k;
                 const uint2 rq = ranges[q];
-                const bool located = rq.y == 0xFFFFFFFFu;                              // already a text position (fm_match_locate_one)
-                const uint32_t full = located ? 1u : ((rq.x <= rq.y) ? (rq.y - rq.x + 1u) : 0u);
-                const uint32_t sz = full < g.max_seed_hits ? full : g.max_seed_hits;
+                const uint32_t sz = seed_range_size(rq, g.max_seed_hits);
                 if (sz == 0u) continue;
+                const bool located = rq.y == 0xFFFFFFFFu;                              // already a text position (fm_match_locate_one)
                 const uint32_t base = run, x = rq.x, seed_begin = k * g.seed_interval;
                 run += sz;
                 for (uint32_t j = 0; j < sz; ++j) {
                     const uint32_t h = base + j;
                     if (h >= kept) break;                                              // beyond the caller's capacity
-                    const uint32_t pos = located ? x : fm_locate_one(f, x + j);
-                    const uint32_t diag = pos > seed_begin ? pos - seed_begin : 0u;
-                    const uint32_t gb = diag > g.band / 2u ? diag - g.band / 2u : 0u;
-                    const uint64_t ge64 = (uint64_t)gb + len + g.band;
-                    const uint32_t ge = ge64 < g.genome_len ? (uint32_t)ge64 : g.genome_len;
+                    const uint2 w = hit_window(located ? x : fm_locate_one(f, x + j), seed_begin, len, g.band, g.genome_len);
+                    const uint32_t gb = w.x, ge = w.y;
                     bool seen = false;
 #pragma unroll
                     for (int e = 0; e < RJ_LOCAL; ++e) seen |= (e < n_local) && lk_s[e] == s && lk_b[e] == gb && lk_e[e] == ge;
@@ -390,10 +379,8 @@ pipe_reduce_jobs_kernel(const PipeGeom g, const uint32_t* __restrict__ counts, c
                         const int32_t* __restrict__ job_score, unsigned long long* __restrict__ best_key)
 {
     const uint32_t n = counts[2];
-    for (uint32_t j = blockIdx.x * 256 + threadIdx.x; j < n; j += gridDim.x * 256) {
-        const unsigned long long key = ((unsigned long long)((uint32_t)job_score[j] ^ 0x80000000u) << 32) | (unsigned long long)(0xFFFFFFFFu - j_first[j]);
-        atomicMax(best_key + j_string[j] / g.strands, key);
-    }
+    for (uint32_t j = blockIdx.x * 256 + threadIdx.x; j < n; j += gridDim.x * 256)
+        atomicMax(best_key + j_string[j] / g.strands, nvb::best_key(job_score[j], j_first[j]));
 }
 
 __global__ void __launch_bounds__(256)
@@ -414,8 +401,7 @@ pipe_finalize_jobs_kernel(const PipeGeom g, const uint32_t* __restrict__ counts,
     const uint32_t n = counts[2];
     for (uint32_t j = blockIdx.x * 256 + threadIdx.x; j < n; j += gridDim.x * 256) {
         const uint32_t s = j_string[j], read = s / g.strands;
-        const unsigned long long key = ((unsigned long long)((uint32_t)job_score[j] ^ 0x80000000u) << 32) | (unsigned long long)(0xFFFFFFFFu - j_first[j]);
-        if (best_key[read] != key) continue;
+        if (best_key[read] != nvb::best_key(job_score[j], j_first[j])) continue;
         best_score[read] = job_score[j]; best_pos[read] = jt_off[j] + job_sink[j].x; best_strand[read] = (uint8_t)(s % g.strands);
     }
 }
@@ -491,9 +477,7 @@ pipe_scatter_scores_kernel(const PipeGeom g, const uint32_t* __restrict__ counts
     const int32_t sc = job_score[j];
     score[h] = sc;
     sink[h]  = job_sink[j];
-    const uint32_t read = hit_string[h] / g.strands;
-    const unsigned long long key = ((unsigned long long)((uint32_t)sc ^ 0x80000000u) << 32) | (unsigned long long)(0xFFFFFFFFu - h);
-    atomicMax(best_key + read, key);
+    atomicMax(best_key + hit_string[h] / g.strands, nvb::best_key(sc, h));
 }
 
 // best hit per read: max score, ties -> smallest hit index (deterministic)
@@ -503,9 +487,7 @@ pipe_reduce_kernel(const PipeGeom g, const uint32_t* __restrict__ counts, const 
 {
     const uint32_t h = blockIdx.x * 256 + threadIdx.x;
     if (h >= counts[0]) return;
-    const uint32_t read = hit_string[h] / g.strands;
-    const unsigned long long key = ((unsigned long long)((uint32_t)score[h] ^ 0x80000000u) << 32) | (unsigned long long)(0xFFFFFFFFu - h);
-    atomicMax(best_key + read, key);
+    atomicMax(best_key + hit_string[h] / g.strands, nvb::best_key(score[h], h));
 }
 
 __global__ void __launch_bounds__(256)
@@ -517,8 +499,8 @@ pipe_finalize_kernel(const PipeGeom g, const unsigned long long* __restrict__ be
     if (r >= g.n_reads) return;
     const unsigned long long key = best_key[r];
     if (key == 0ull) { best_score[r] = INT_MIN; best_pos[r] = 0xFFFFFFFFu; if (best_strand) best_strand[r] = 0; return; }
-    const uint32_t h = 0xFFFFFFFFu - (uint32_t)(key & 0xFFFFFFFFull);
-    best_score[r] = (int32_t)((uint32_t)(key >> 32) ^ 0x80000000u);
+    const uint32_t h = best_key_hit(key);
+    best_score[r] = best_key_score(key);
     best_pos[r] = t_off[h] + sink[h].x;
     if (best_strand) best_strand[r] = (uint8_t)(hit_string[h] % g.strands);
 }
@@ -535,7 +517,7 @@ pipe_best_jobs_kernel(const PipeGeom g, const unsigned long long* __restrict__ b
     if (r >= g.n_reads) return;
     const unsigned long long key = best_key[r];
     if (key == 0ull) { bp_off[r] = 0; bp_len[r] = 0; bt_off[r] = 0; bt_len[r] = 0; if (strand) strand[r] = 0; return; }
-    const uint32_t h = 0xFFFFFFFFu - (uint32_t)(key & 0xFFFFFFFFull);
+    const uint32_t h = best_key_hit(key);
     bp_off[r] = p_off[h]; bp_len[r] = p_len[h]; bt_off[r] = t_off[h]; bt_len[r] = t_len[h];
     if (strand) strand[r] = (uint8_t)(hit_string[h] % g.strands);
 }
@@ -686,12 +668,15 @@ pair_finalize_kernel(const uint32_t n_pairs, const nvb_pair_params pp, const uin
 
 using namespace nvb;
 
-// stage boundaries of the most recent nvb_seed_extend call ON EACH DEVICE (events are recorded on the caller's stream; they
+#define PIPE_TRY(expr) do { const int _r = (expr); if (_r != NVB_OK) return _r; } while (0)
+#define PIPE_SIZE_QUERY(expr) do { const int _r = (expr); if (_r != NVB_E_TEMP_SIZE && _r != NVB_OK) return _r; } while (0)
+#define NVB_STAGE(i) do { if (c.ev) NVB_CUDA_TRY(cudaEventRecord(c.ev[i], c.s)); } while (0)
+
+// stage boundaries of the most recent direct nvb_seed_extend* call ON EACH DEVICE (events are recorded on the caller's stream; they
 // cost no synchronisation).  [0]=start, then after: strings, seed match, slots, locate+windows, job dedup, extension, reduce.
-// Events belong to the device that created them, so the set is per device, created under a mutex on first use; a host that
-// drives several GPUs from one process (one compute thread per device) gets one set per GPU.  Callers that run several
-// batches of one device concurrently (nvb_pipeline) pass their own events instead.
-struct StageEvents { cudaEvent_t ev[8]; bool ready, valid; };
+// Events belong to the device that created them, so the set is per device, created under a mutex on first use; a host that drives
+// several GPUs from one process (one compute thread per device) gets one set per GPU.  nvb_pipeline's batches record none.
+struct StageEvents { cudaEvent_t ev[8]; bool ready; std::atomic<bool> valid; };
 static StageEvents g_stage[NVB_MAX_DEVICES];
 static std::mutex  g_stage_mutex;
 static int default_stage_events(StageEvents** out)
@@ -708,32 +693,324 @@ static int default_stage_events(StageEvents** out)
     *out = &S;
     return NVB_OK;
 }
-#define NVB_STAGE(i) do { NVB_CUDA_TRY(cudaEventRecord(SE->ev[i], s)); } while (0)
 
 extern "C" int nvb_seed_extend_stage_ms(float ms[7])
 {
     if (!ms) return NVB_E_INVALID;
     StageEvents* SE = nullptr;
-    { const int r = default_stage_events(&SE); if (r != NVB_OK) return r; }
-    if (!SE->valid) return NVB_E_INVALID;
+    PIPE_TRY(default_stage_events(&SE));
+    if (!SE->valid.load(std::memory_order_acquire)) return NVB_E_INVALID;
     NVB_CUDA_TRY(cudaEventSynchronize(SE->ev[7]));
     for (int i = 0; i < 7; ++i) NVB_CUDA_TRY(cudaEventElapsedTime(&ms[i], SE->ev[i], SE->ev[i + 1]));
     return NVB_OK;
 }
 
-static int g_perfect_shortcut = 1;     // 0 = every alignment job through the DP kernels (nvb_debug_perfect_shortcut)
-static int g_seed_split = 1;           // 0 = the located seed match in one pass (nvb_debug_seed_split)
-static int g_pipe_path = 0;            // 0 = automatic, 1 = always the per-hit path, 2 = per-read path without the in-kernel locate (nvb_debug_pipeline_path)
+// test / tuning switches (include/nvbio_b200_debug.h); a call reads each of them once
+static std::atomic<int> g_perfect_shortcut{1};     // 0 = every alignment job through the DP kernels
+static std::atomic<int> g_seed_split{1};           // 0 = the located seed match in one pass
+static std::atomic<int> g_pipe_path{0};            // 0 = automatic, 1 = always the per-hit path
+extern "C" void nvb_debug_pipeline_path(int path) { g_pipe_path.store(path, std::memory_order_relaxed); }
+extern "C" void nvb_debug_seed_split(int on) { g_seed_split.store(on, std::memory_order_relaxed); }
+extern "C" void nvb_debug_perfect_shortcut(int on) { g_perfect_shortcut.store(on, std::memory_order_relaxed); }
 
-static int seed_extend_impl(const nvb_fm_index* fmi, const uint32_t* d_genome,
-                    const nvb_string_set* reads, uint32_t n_reads,
-                    const nvb_seed_extend_params* P, uint32_t hit_capacity,
-                    int32_t* d_best_score, uint32_t* d_best_pos,
-                    uint32_t* d_n_hits, uint32_t* d_hit_read, nvb_uint2* d_hit_window,
-                    int32_t* d_hit_score, nvb_uint2* d_hit_sink,
-                    const nvb_best_alignment_out* BA,
-                    const nvb_pair_params* PP, const nvb_pair_out* PO,
-                    void* d_temp, size_t* temp_bytes, void* stream)
+// grids of kernels striding over a job count that lives on the device: resident CTAs of the 148 SMs, not hit_capacity / 256 mostly empty ones
+constexpr uint32_t SHORTCUT_GRID_CAP = 148u * 8u;
+constexpr uint32_t REDUCE_GRID_CAP   = 148u * 16u;
+
+// an alignment job list: pattern = symbols [p_off, + p_len) of the [fw,rc] strings, text = genome [t_off, + t_len)
+struct JobList { uint32_t *p_off, *p_len, *t_off, *t_len; };
+static JobList take_jobs(TempCarver& tc, size_t n) { return JobList{tc.take<uint32_t>(n), tc.take<uint32_t>(n), tc.take<uint32_t>(n), tc.take<uint32_t>(n)}; }
+
+// the path of one call, decided once
+struct PipePlan {
+    bool dedup;        // identical (string, window) jobs of a read are scored once
+    bool per_read;     // no per-hit output wanted: distinct jobs straight from a thread per read, no per-hit array at all
+    bool eligible;     // the per-read jobs qualify for the gapless shortcut (its arrays are carved)
+    bool shortcut;     // ... and take it
+    bool locate;       // the seed match locates single-row ranges (per-read path on an index with the full suffix array)
+    bool split;        // ... in two passes (a k-mer table shorter than the seed)
+};
+
+// the temp arrays of one call, in carve order; those of a path the call does not take stay null
+struct PipeTemp {
+    uint32_t *str_words, *str_len; uint8_t* str_quals; uint2* ranges; uint32_t *sizes, *excl, *counts, *seed_todo_n;   // counts: hits kept, found, unique jobs
+    uint32_t *j_string, *j_first, *leader, *flag, *job_idx;            // per-read path: string, first hit of every job; per-hit de-duplication
+    JobList jobs; int32_t* job_score; uint2* job_sink;                  // the unique jobs (de-duplication)
+    JobList dp; uint32_t* dp_job; int32_t* dp_score; uint2* dp_sink; uint32_t* dp_count;    // jobs the gapless shortcut leaves to the DP
+    uint32_t* hit_string; JobList hits; int32_t* h_score; uint2* h_sink;    // per-hit path
+    unsigned long long* best_key; uint8_t* rb_strand; char *scan_tmp, *gotoh_tmp; size_t scan_bytes, gotoh_bytes;
+    JobList best; int32_t* b_score; uint2 *b_sink, *b_source; char* tb_tmp; size_t tb_bytes;    // best-alignment traceback
+    uint32_t *pw_want, *pw_idx, *pw_pstr, *pw_toff, *pw_tlen, *pcounts;                         // paired-end rescue
+    JobList rescue; int32_t* rs_score; uint2* rs_sink; char *pscan_tmp, *full_tmp; size_t pscan_bytes, full_bytes;
+};
+
+struct PipeCall {
+    const nvb_seed_extend_params* P; PipeGeom g; uint32_t nq, spw, hit_capacity; FmIndex f; StrSet rd; const uint32_t* genome;
+    nvb_string_set pats, txts;          // job-list views: formats and maximum lengths (their pointers are placeholders, see job_views)
+    PipePlan plan; PipeTemp t;
+    cudaStream_t s; cudaEvent_t* ev;                    // ev: stage events to record, or null
+};
+
+static void job_views(const PipeCall& c, const JobList& j, nvb_string_set& pats, nvb_string_set& txts)
+{
+    pats = c.pats; pats.d_words = c.t.str_words; pats.d_offsets = j.p_off; pats.d_lengths = j.p_len;
+    txts = c.txts; txts.d_words = c.genome;      txts.d_offsets = j.t_off; txts.d_lengths = j.t_len;
+}
+
+// the banded extension of a job list whose length lives on the device
+static int score_jobs(const PipeCall& c, const JobList& j, const uint32_t* d_n_jobs, int32_t* score, uint2* sink)
+{
+    nvb_string_set pats, txts;
+    job_views(c, j, pats, txts);
+    size_t gb = c.t.gotoh_bytes;
+    return nvb_banded_gotoh_score_indirect(c.P->band_len, c.P->type, &c.P->scheme, &pats, c.t.str_quals, &txts, d_n_jobs, c.hit_capacity,
+                                           score, (nvb_uint2*)sink, c.t.gotoh_tmp, &gb, c.s);
+}
+
+// carves the temp arrays (the layout behind *temp_bytes) and queries the temp the library calls of the stages need
+static int carve_temp(PipeCall& c, TempCarver& tc, int32_t* d_hit_score, nvb_uint2* d_hit_sink,
+                      const nvb_best_alignment_out* BA, const nvb_pair_params* PP)
+{
+    const nvb_seed_extend_params* P = c.P;
+    const PipeGeom& g = c.g; const PipePlan& pl = c.plan; PipeTemp& t = c.t;
+    const uint32_t cap = c.hit_capacity, n_reads = g.n_reads;
+    PIPE_SIZE_QUERY(nvb_banded_gotoh_score(P->band_len, P->type, &P->scheme, &c.pats, nullptr, &c.txts, cap, (int32_t*)16, (nvb_uint2*)16, nullptr,
+                                           &t.gotoh_bytes, c.s));
+    t.str_words = tc.take<uint32_t>((size_t)g.n_strings * (g.stride / c.spw) + 4);
+    t.str_len   = tc.take<uint32_t>(g.n_strings);
+    t.str_quals = P->d_read_quals ? tc.take<uint8_t>((size_t)g.n_strings * g.stride + 16) : nullptr;
+    t.ranges    = tc.take<uint2>(c.nq);
+    t.sizes     = tc.take<uint32_t>(c.nq);
+    t.excl      = tc.take<uint32_t>((size_t)c.nq + (SEED_TODO_LISTS + 1u) * SEED_BLOCK * SEED_ITER);   // (+ slack: before the scan it holds the seed-match todo lists)
+    t.counts    = tc.take<uint32_t>(4);
+    t.seed_todo_n = tc.take<uint32_t>(SEED_TODO_LISTS * SEED_TODO_PITCH);
+    if (pl.per_read) { t.j_string = tc.take<uint32_t>(cap); t.j_first = tc.take<uint32_t>(cap); }
+    if (pl.dedup && !pl.per_read) { t.leader = tc.take<uint32_t>(cap); t.flag = tc.take<uint32_t>(cap); t.job_idx = tc.take<uint32_t>(cap); }
+    if (pl.dedup) { t.jobs = take_jobs(tc, cap); t.job_score = tc.take<int32_t>(cap); t.job_sink = tc.take<uint2>(cap); }
+    if (pl.eligible) {
+        t.dp = take_jobs(tc, cap); t.dp_job = tc.take<uint32_t>(cap); t.dp_score = tc.take<int32_t>(cap); t.dp_sink = tc.take<uint2>(cap); t.dp_count = tc.take<uint32_t>(4);
+    }
+    if (!pl.per_read) {
+        t.hit_string = tc.take<uint32_t>(cap); t.hits = take_jobs(tc, cap);
+        t.h_score = d_hit_score ? d_hit_score : tc.take<int32_t>(cap); t.h_sink = d_hit_sink ? (uint2*)d_hit_sink : tc.take<uint2>(cap);
+    }
+    t.best_key = tc.take<unsigned long long>(n_reads); t.rb_strand = tc.take<uint8_t>((size_t)n_reads + 16);
+    NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, t.scan_bytes, t.sizes, t.excl, (int)c.nq, c.s));
+    if (pl.dedup && !pl.per_read && cap) {
+        size_t scan2_bytes = 0;
+        NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan2_bytes, t.flag, t.job_idx, (int)cap, c.s));
+        if (scan2_bytes > t.scan_bytes) t.scan_bytes = scan2_bytes;
+    }
+    t.scan_tmp = tc.take<char>(t.scan_bytes); t.gotoh_tmp = tc.take<char>(t.gotoh_bytes);
+    if (BA) {               // best-alignment traceback: per-read job arrays + the traceback's own temp (direction matrices)
+        t.best = take_jobs(tc, n_reads);
+        t.b_score = tc.take<int32_t>(n_reads); t.b_sink = tc.take<uint2>(n_reads); t.b_source = tc.take<uint2>(n_reads);
+        PIPE_SIZE_QUERY(nvb_banded_gotoh_traceback(P->band_len, P->type, &P->scheme, &c.pats, nullptr, &c.txts, n_reads, nullptr, nullptr, nullptr, nullptr,
+                                                   BA->max_ops, nullptr, nullptr, &t.tb_bytes, c.s));
+        t.tb_tmp = tc.take<char>(t.tb_bytes);
+    }
+    if (PP) {               // paired-end stage: job slots (2 per pair), compacted full-DP jobs and the DP's own temp
+        const uint32_t pcap = PP->rescue_capacity;
+        t.pw_want = tc.take<uint32_t>(n_reads); t.pw_idx = tc.take<uint32_t>(n_reads); t.pw_pstr = tc.take<uint32_t>(n_reads);
+        t.pw_toff = tc.take<uint32_t>(n_reads); t.pw_tlen = tc.take<uint32_t>(n_reads); t.pcounts = tc.take<uint32_t>(4);
+        t.rescue = take_jobs(tc, pcap); t.rs_score = tc.take<int32_t>(pcap); t.rs_sink = tc.take<uint2>(pcap);
+        NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, t.pscan_bytes, t.pw_want, t.pw_idx, (int)n_reads, c.s));
+        t.pscan_tmp = tc.take<char>(t.pscan_bytes);
+        nvb_string_set rtxts = c.txts; rtxts.length = PP->max_frag;
+        PIPE_SIZE_QUERY(nvb_gotoh_score_indirect(P->type, &P->scheme, &c.pats, nullptr, &rtxts, (const uint32_t*)16, pcap, (int32_t*)16, (nvb_uint2*)16,
+                                                 nullptr, &t.full_bytes, c.s));
+        t.full_tmp = tc.take<char>(t.full_bytes);
+    }
+    return NVB_OK;
+}
+
+// 1. [fw, rc] strings (and their base qualities)
+static int run_strings(const PipeCall& c)
+{
+    const PipeGeom& g = c.g; const PipeTemp& t = c.t;
+    const uint64_t total_words = (uint64_t)g.n_strings * (g.stride / c.spw);
+    const uint32_t grid = (uint32_t)((total_words + 255) / 256);
+    if (g.bits == 2 && c.rd.big_endian) pipe_make_strings_2bit_be_kernel<<<grid, 256, 0, c.s>>>(c.rd, g, t.str_words, t.str_len);
+    else if (g.bits == 2)               pipe_make_strings_kernel<2><<<grid, 256, 0, c.s>>>(c.rd, g, t.str_words, t.str_len);
+    else                                pipe_make_strings_kernel<4><<<grid, 256, 0, c.s>>>(c.rd, g, t.str_words, t.str_len);
+    NVB_LAUNCH_CHECK();
+    if (t.str_quals) {
+        const uint64_t total = (uint64_t)g.n_strings * g.stride;
+        pipe_make_quals_kernel<<<(uint32_t)((total + 255) / 256), 256, 0, c.s>>>(c.rd, g, c.P->d_read_quals, t.str_quals);
+        NVB_LAUNCH_CHECK();
+    }
+    return NVB_OK;
+}
+
+// 2. seed ranges
+static int run_seed_match(const PipeCall& c)
+{
+    const PipeGeom& g = c.g; const PipeTemp& t = c.t;
+    const uint32_t grid = (c.nq + SEED_BLOCK - 1) / SEED_BLOCK;
+    const uint32_t* loc_genome = c.plan.locate ? c.genome : nullptr;
+    if (c.plan.split) {
+        // seeds on k-mers with >= 3 occurrences are finished by a second kernel (the lists live in `excl`, which the hit-slot scan overwrites)
+        NVB_CUDA_TRY(cudaMemsetAsync(t.seed_todo_n, 0, SEED_TODO_LISTS * SEED_TODO_PITCH * sizeof(uint32_t), c.s));
+        const uint32_t grid1 = (grid + SEED_ITER - 1u) / SEED_ITER;
+        if (g.bits == 2) pipe_seed_match_kernel<2, true><<<grid1, SEED_BLOCK, 0, c.s>>>(c.f, g, t.str_words, t.str_len, loc_genome, t.ranges, t.sizes, t.excl, t.seed_todo_n);
+        else             pipe_seed_match_kernel<4, true><<<grid1, SEED_BLOCK, 0, c.s>>>(c.f, g, t.str_words, t.str_len, loc_genome, t.ranges, t.sizes, t.excl, t.seed_todo_n);
+        NVB_LAUNCH_CHECK();
+        const uint32_t wgrid = SEED_TODO_LISTS * 37u;                                  // 2368 CTAs = 148 SMs x 16 resident CTAs
+        if (g.bits == 2) pipe_seed_match_wide_kernel<2><<<wgrid, SEED_BLOCK, 0, c.s>>>(c.f, g, t.str_words, loc_genome, t.ranges, t.sizes, t.excl, t.seed_todo_n, grid1);
+        else             pipe_seed_match_wide_kernel<4><<<wgrid, SEED_BLOCK, 0, c.s>>>(c.f, g, t.str_words, loc_genome, t.ranges, t.sizes, t.excl, t.seed_todo_n, grid1);
+    } else {
+        if (g.bits == 2) pipe_seed_match_kernel<2, false><<<grid, SEED_BLOCK, 0, c.s>>>(c.f, g, t.str_words, t.str_len, loc_genome, t.ranges, t.sizes, nullptr, nullptr);
+        else             pipe_seed_match_kernel<4, false><<<grid, SEED_BLOCK, 0, c.s>>>(c.f, g, t.str_words, t.str_len, loc_genome, t.ranges, t.sizes, nullptr, nullptr);
+    }
+    NVB_LAUNCH_CHECK();
+    return NVB_OK;
+}
+
+// 3. hit slots
+static int run_hit_slots(const PipeCall& c)
+{
+    size_t sb = c.t.scan_bytes; NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(c.t.scan_tmp, sb, c.t.sizes, c.t.excl, (int)c.nq, c.s));
+    pipe_count_kernel<<<1, 32, 0, c.s>>>(c.t.excl, c.t.sizes, c.nq, c.hit_capacity, c.t.counts);
+    NVB_LAUNCH_CHECK();
+    return NVB_OK;
+}
+
+// 4'. per read: locate, window, distinct jobs; 5'. extension; 6'. best job per read
+static int run_per_read(const PipeCall& c, int32_t* d_best_score, uint32_t* d_best_pos)
+{
+    const PipeGeom& g = c.g; const PipeTemp& t = c.t;
+    const uint32_t cap = c.hit_capacity, hgrid = (cap + 255) / 256;
+    NVB_CUDA_TRY(cudaMemsetAsync(t.counts + 2, 0, sizeof(uint32_t), c.s));
+    NVB_CUDA_TRY(cudaMemsetAsync(t.best_key, 0, sizeof(unsigned long long) * g.n_reads, c.s));
+    if (cap) {
+        pipe_read_jobs_kernel<<<(g.n_reads + RJ_BLOCK - 1) / RJ_BLOCK, RJ_BLOCK, 0, c.s>>>(c.f, g, t.ranges, t.sizes, t.excl, t.str_len, t.counts, t.j_string,
+                                                                                         t.j_first, t.jobs.p_off, t.jobs.p_len, t.jobs.t_off, t.jobs.t_len);
+        NVB_LAUNCH_CHECK();
+    }
+    NVB_STAGE(4); NVB_STAGE(5);                         // (the jobs come out distinct: no de-duplication stage)
+    if (cap && c.plan.shortcut) {
+        const uint32_t jgrid = hgrid < SHORTCUT_GRID_CAP ? hgrid : SHORTCUT_GRID_CAP;
+        const nvb_gotoh_scheme& SC = c.P->scheme;
+        NVB_CUDA_TRY(cudaMemsetAsync(t.dp_count, 0, sizeof(uint32_t), c.s));
+        pipe_perfect_jobs_kernel<<<jgrid, 256, 0, c.s>>>(g, SC.match, SC.mismatch, SC.pattern_gap_open > SC.text_gap_open ? SC.pattern_gap_open : SC.text_gap_open,
+                                                         t.counts, t.str_words, c.genome, t.jobs.p_off, t.jobs.p_len, t.jobs.t_off, t.jobs.t_len,
+                                                         t.job_score, t.job_sink, t.dp.p_off, t.dp.p_len, t.dp.t_off, t.dp.t_len, t.dp_job, t.dp_count);
+        NVB_LAUNCH_CHECK();
+        PIPE_TRY(score_jobs(c, t.dp, t.dp_count, t.dp_score, t.dp_sink));
+        pipe_scatter_dp_kernel<<<jgrid, 256, 0, c.s>>>(t.dp_count, t.dp_job, t.dp_score, t.dp_sink, t.job_score, t.job_sink);
+        NVB_LAUNCH_CHECK();
+    } else if (cap) PIPE_TRY(score_jobs(c, t.jobs, t.counts + 2, t.job_score, t.job_sink));
+    NVB_STAGE(6);
+    pipe_init_best_kernel<<<(g.n_reads + 255) / 256, 256, 0, c.s>>>(g.n_reads, d_best_score, d_best_pos, t.rb_strand);
+    NVB_LAUNCH_CHECK();
+    if (cap) {
+        const uint32_t jgrid = hgrid < REDUCE_GRID_CAP ? hgrid : REDUCE_GRID_CAP;
+        pipe_reduce_jobs_kernel<<<jgrid, 256, 0, c.s>>>(g, t.counts, t.j_string, t.j_first, t.job_score, t.best_key);
+        NVB_LAUNCH_CHECK();
+        pipe_finalize_jobs_kernel<<<jgrid, 256, 0, c.s>>>(g, t.counts, t.j_string, t.j_first, t.jobs.t_off, t.job_score, t.job_sink, t.best_key,
+                                                          d_best_score, d_best_pos, t.rb_strand);
+        NVB_LAUNCH_CHECK();
+    }
+    return NVB_OK;
+}
+
+// 4. locate + windows per hit; 4b. collapse identical (string, window) jobs; 5. extension; 6. best hit per read; the hit arrays
+static int run_per_hit(const PipeCall& c, int32_t* d_best_score, uint32_t* d_best_pos, uint32_t* d_hit_read, nvb_uint2* d_hit_window)
+{
+    const PipeGeom& g = c.g; const PipeTemp& t = c.t;
+    const uint32_t cap = c.hit_capacity, hgrid = (cap + 255) / 256;
+    const bool dedup = c.plan.dedup;
+    if (cap) {
+        pipe_expand_hits_kernel<<<(c.nq + 255) / 256, 256, 0, c.s>>>(c.f, g, t.ranges, t.sizes, t.excl, t.str_len, t.counts, t.hit_string, t.hits.p_off, t.hits.p_len,
+                                                                     t.hits.t_off, t.hits.t_len);
+        NVB_LAUNCH_CHECK();
+    }
+    NVB_STAGE(4);
+    if (dedup && cap) {
+        pipe_find_leaders_kernel<<<hgrid, 256, 0, c.s>>>(t.counts, t.hit_string, t.hits.t_off, t.hits.t_len, t.leader, t.flag);
+        NVB_LAUNCH_CHECK();
+        // the scan runs over the whole capacity; job_idx[h] depends only on flag[0..h), so the (unwritten) entries
+        // past counts[0] cannot influence any index that is read back
+        size_t sb = t.scan_bytes; NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(t.scan_tmp, sb, t.flag, t.job_idx, (int)cap, c.s));
+        pipe_job_count_kernel<<<1, 32, 0, c.s>>>(t.job_idx, t.flag, t.counts);
+        NVB_LAUNCH_CHECK();
+        pipe_compact_jobs_kernel<<<hgrid, 256, 0, c.s>>>(t.counts, t.flag, t.job_idx, t.hits.p_off, t.hits.p_len, t.hits.t_off, t.hits.t_len,
+                                                         t.jobs.p_off, t.jobs.p_len, t.jobs.t_off, t.jobs.t_len);
+        NVB_LAUNCH_CHECK();
+    }
+    NVB_STAGE(5);
+    NVB_CUDA_TRY(cudaMemsetAsync(t.best_key, 0, sizeof(unsigned long long) * g.n_reads, c.s));
+    if (cap && dedup) {
+        PIPE_TRY(score_jobs(c, t.jobs, t.counts + 2, t.job_score, t.job_sink));
+        pipe_scatter_scores_kernel<<<hgrid, 256, 0, c.s>>>(g, t.counts, t.leader, t.job_idx, t.job_score, t.job_sink, t.hit_string, t.h_score, t.h_sink, t.best_key);
+        NVB_LAUNCH_CHECK();
+    } else if (cap) PIPE_TRY(score_jobs(c, t.hits, t.counts, t.h_score, t.h_sink));
+    NVB_STAGE(6);
+    if (cap && !dedup) {                                // (with job de-duplication the scatter kernel did the reduction)
+        pipe_reduce_kernel<<<hgrid, 256, 0, c.s>>>(g, t.counts, t.hit_string, t.h_score, t.best_key);
+        NVB_LAUNCH_CHECK();
+    }
+    pipe_finalize_kernel<<<(g.n_reads + 255) / 256, 256, 0, c.s>>>(g, t.best_key, t.hits.t_off, t.h_sink, t.hit_string, d_best_score, d_best_pos, t.rb_strand);
+    NVB_LAUNCH_CHECK();
+    if (cap && (d_hit_read || d_hit_window)) {
+        pipe_export_hits_kernel<<<hgrid, 256, 0, c.s>>>(g, t.counts, t.hit_string, t.hits.t_off, t.hits.t_len, d_hit_read, (uint2*)d_hit_window);
+        NVB_LAUNCH_CHECK();
+    }
+    return NVB_OK;
+}
+
+// the alignment (ops, begin, strand) of every read's best hit (per-hit path)
+static int run_traceback(const PipeCall& c, const nvb_best_alignment_out* BA)
+{
+    const PipeGeom& g = c.g; const PipeTemp& t = c.t;
+    const uint32_t rgrid = (g.n_reads + 255) / 256;
+    pipe_best_jobs_kernel<<<rgrid, 256, 0, c.s>>>(g, t.best_key, t.hit_string, t.hits.p_off, t.hits.p_len, t.hits.t_off, t.hits.t_len,
+                                                  t.best.p_off, t.best.p_len, t.best.t_off, t.best.t_len, BA->d_strand);
+    NVB_LAUNCH_CHECK();
+    nvb_string_set pats, txts;
+    job_views(c, t.best, pats, txts);
+    size_t tbb = t.tb_bytes;
+    PIPE_TRY(nvb_banded_gotoh_traceback(c.P->band_len, c.P->type, &c.P->scheme, &pats, t.str_quals, &txts, g.n_reads, t.b_score, (nvb_uint2*)t.b_sink,
+                                        (nvb_uint2*)t.b_source, BA->d_ops, BA->max_ops, BA->d_n_ops, t.tb_tmp, &tbb, c.s));
+    pipe_best_begin_kernel<<<rgrid, 256, 0, c.s>>>(g, t.best_key, t.best.t_off, t.b_source, BA->d_n_ops, (uint2*)BA->d_begin);
+    NVB_LAUNCH_CHECK();
+    return NVB_OK;
+}
+
+// paired-end stage: concordance of the mates' best alignments, full-DP rescue of the opposite mate for the others
+static int run_paired(const PipeCall& c, const nvb_pair_params* PP, const nvb_pair_out* PO, int32_t* d_best_score, uint32_t* d_best_pos)
+{
+    const PipeGeom& g = c.g; const PipeTemp& t = c.t;
+    const uint32_t n_reads = g.n_reads, n_pairs = n_reads / 2u, cap = PP->rescue_capacity;
+    const uint32_t pgrid = (n_pairs + 255) / 256, sgrid = (n_reads + 255) / 256;
+    pair_classify_kernel<<<pgrid, 256, 0, c.s>>>(g, n_pairs, *PP, d_best_score, d_best_pos, t.rb_strand, t.str_len, t.pw_want, t.pw_pstr, t.pw_toff, t.pw_tlen,
+                                                 PO->d_pair_score, PO->d_pair_flags, PO->d_mate_score, PO->d_mate_pos, PO->d_mate_strand);
+    NVB_LAUNCH_CHECK();
+    size_t sb = t.pscan_bytes; NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(t.pscan_tmp, sb, t.pw_want, t.pw_idx, (int)n_reads, c.s));
+    pair_job_count_kernel<<<1, 32, 0, c.s>>>(t.pw_idx, t.pw_want, n_reads, cap, t.pcounts);
+    NVB_LAUNCH_CHECK();
+    if (cap) {
+        pair_compact_kernel<<<sgrid, 256, 0, c.s>>>(g, n_reads, cap, t.pw_want, t.pw_idx, t.pw_pstr, t.pw_toff, t.pw_tlen, t.str_len,
+                                                    t.rescue.p_off, t.rescue.p_len, t.rescue.t_off, t.rescue.t_len);
+        NVB_LAUNCH_CHECK();
+        nvb_string_set pats, txts;
+        job_views(c, t.rescue, pats, txts);
+        txts.length = PP->max_frag; size_t fb = t.full_bytes;
+        PIPE_TRY(nvb_gotoh_score_indirect(c.P->type, &c.P->scheme, &pats, t.str_quals, &txts, t.pcounts, cap, t.rs_score, (nvb_uint2*)t.rs_sink,
+                                          t.full_tmp, &fb, c.s));
+    }
+    pair_finalize_kernel<<<pgrid, 256, 0, c.s>>>(n_pairs, *PP, t.pw_want, t.pw_idx, t.pw_toff, t.rs_score, t.rs_sink, PO->d_pair_score, PO->d_pair_flags,
+                                                 PO->d_mate_score, PO->d_mate_pos, PO->d_mate_strand);
+    NVB_LAUNCH_CHECK();
+    if (PO->d_n_rescue) NVB_CUDA_TRY(cudaMemcpyAsync(PO->d_n_rescue, t.pcounts, 2 * sizeof(uint32_t), cudaMemcpyDeviceToDevice, c.s));
+    return NVB_OK;
+}
+
+int nvb::seed_extend_impl(const nvb_fm_index* fmi, const uint32_t* d_genome, const nvb_string_set* reads, uint32_t n_reads,
+                          const nvb_seed_extend_params* P, uint32_t hit_capacity, int32_t* d_best_score, uint32_t* d_best_pos,
+                          uint32_t* d_n_hits, uint32_t* d_hit_read, nvb_uint2* d_hit_window, int32_t* d_hit_score, nvb_uint2* d_hit_sink,
+                          const nvb_best_alignment_out* BA, const nvb_pair_params* PP, const nvb_pair_out* PO,
+                          void* d_temp, size_t* temp_bytes, void* stream, bool record_stages)
 {
     if (PP) {
         if (!PO || !PO->d_pair_score || !PO->d_pair_flags || !PO->d_mate_score || !PO->d_mate_pos || !PO->d_mate_strand) return NVB_E_INVALID;
@@ -747,358 +1024,80 @@ static int seed_extend_impl(const nvb_fm_index* fmi, const uint32_t* d_genome,
     const uint32_t max_len = reads->length;                 // maximum read length (== length for fixed-length sets)
     if (max_len < P->seed_len) return NVB_E_INVALID;
 
-    PipeGeom g;
+    PipeCall c{};
+    PipeGeom& g = c.g;
     g.n_reads = n_reads; g.strands = P->both_strands ? 2u : 1u; g.n_strings = n_reads * g.strands;
-    g.bits = reads->bits;
-    const uint32_t spw = 32u / g.bits;
-    g.stride = (max_len + spw - 1u) / spw * spw;
+    g.bits = reads->bits; c.spw = 32u / g.bits;
+    g.stride = (max_len + c.spw - 1u) / c.spw * c.spw;
     g.seeds_per_string = (max_len - P->seed_len) / P->seed_interval + 1u;
     g.seed_len = P->seed_len; g.seed_interval = P->seed_interval; g.band = P->band_len;
     g.max_seed_hits = P->max_seed_hits; g.genome_len = fmi->length; g.hit_capacity = hit_capacity;
     if ((uint64_t)g.n_strings * g.stride > 0xFFFFFFFFull) return NVB_E_UNSUPPORTED;
     const uint64_t nq64 = (uint64_t)g.n_strings * g.seeds_per_string;
     if (nq64 > 0x7FFFFFFFull) return NVB_E_UNSUPPORTED;
-    const uint32_t nq = (uint32_t)nq64;
     // hit slots are a uint32 exclusive sum of the clamped range sizes: the worst case must fit
     if (nq64 * (uint64_t)P->max_seed_hits > 0xFFFFFFFFull) return NVB_E_UNSUPPORTED;
-
-    // the extension's own temp requirement
-    nvb_string_set pats, txts;
-    pats.bits = g.bits; pats.big_endian = 1; pats.stride = 0; pats.length = max_len;
-    txts.bits = 2; txts.big_endian = 1; txts.stride = 0; txts.length = max_len + P->band_len;
-    pats.d_words = (const uint32_t*)16; txts.d_words = d_genome;     // placeholders for the size query
-    pats.d_offsets = pats.d_lengths = txts.d_offsets = txts.d_lengths = nullptr;
-    size_t gotoh_bytes = 0;
-    {
-        const int r = nvb_banded_gotoh_score(P->band_len, P->type, &P->scheme, &pats, nullptr, &txts, hit_capacity,
-                                             (int32_t*)16, (nvb_uint2*)16, nullptr, &gotoh_bytes, stream);
-        if (r != NVB_E_TEMP_SIZE && r != NVB_OK) return r;
-    }
-
-    TempCarver tc(d_temp);
-    uint32_t* str_words  = tc.take<uint32_t>((size_t)g.n_strings * (g.stride / spw) + 4);
-    uint32_t* str_len_   = tc.take<uint32_t>(g.n_strings);
-    uint8_t*  str_quals  = P->d_read_quals ? tc.take<uint8_t>((size_t)g.n_strings * g.stride + 16) : nullptr;
-    uint2*    ranges     = tc.take<uint2>(nq);
-    uint32_t* sizes      = tc.take<uint32_t>(nq);
-    uint32_t* excl       = tc.take<uint32_t>((size_t)nq + (SEED_TODO_LISTS + 1u) * SEED_BLOCK * SEED_ITER);   // (+ slack: before the scan it holds the seed-match todo lists)
-    uint32_t* counts     = tc.take<uint32_t>(4);          // [0] hits kept, [1] hits found, [2] unique alignment jobs
-    uint32_t* seed_todo_n = tc.take<uint32_t>(SEED_TODO_LISTS * SEED_TODO_PITCH);
-    const bool dedup = P->dedup_jobs != 0;
-    // per-read path: nobody asked for per-hit outputs, so no per-hit array needs to exist
-    const bool per_read = dedup && g_pipe_path != 1 && !d_hit_read && !d_hit_window && !d_hit_score && !d_hit_sink && !BA;
-    uint32_t* j_string = per_read ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* j_first  = per_read ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* leader  = (dedup && !per_read) ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* flag    = (dedup && !per_read) ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* job_idx = (dedup && !per_read) ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* jp_off  = dedup ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* jp_len  = dedup ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* jt_off  = dedup ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* jt_len  = dedup ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    int32_t*  job_score = dedup ? tc.take<int32_t>(hit_capacity) : nullptr;
-    uint2*    job_sink  = dedup ? tc.take<uint2>(hit_capacity) : nullptr;
+    c.nq = (uint32_t)nq64; c.P = P; c.hit_capacity = hit_capacity; c.f = make_fmindex(fmi); c.rd = make_strset(reads); c.genome = d_genome;
+    c.s = as_stream(stream);
+    c.pats = nvb_string_set{(const uint32_t*)16, g.bits, 1, nullptr, nullptr, 0, max_len};      // (placeholder words for the size queries)
+    c.txts = nvb_string_set{d_genome, 2, 1, nullptr, nullptr, 0, max_len + P->band_len};
+    // the path, decided once
+    PipePlan& p = c.plan;
+    p.dedup = P->dedup_jobs != 0;
+    p.per_read = p.dedup && g_pipe_path.load(std::memory_order_relaxed) != 1 && !(d_hit_read || d_hit_window || d_hit_score || d_hit_sink || BA);
     // exact shortcut for reads that equal their window (pipe_perfect_jobs_kernel): the DP then runs over a compacted job list
-    const nvb_gotoh_scheme& SC = P->scheme;
-    const bool eligible = per_read && P->type == NVB_LOCAL && g.bits == 2 && P->band_len <= 32 && !SC.d_qual_table && SC.match > 0 && SC.mismatch < 0 &&
-                          SC.pattern_gap_open < 0 && SC.pattern_gap_ext <= 0 && SC.text_gap_open < 0 && SC.text_gap_ext <= 0;
-    const bool shortcut = eligible && g_perfect_shortcut;              // (the debug switch does not change the temp layout)
-    uint32_t* dp_p_off = eligible ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* dp_p_len = eligible ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* dp_t_off = eligible ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* dp_t_len = eligible ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    uint32_t* dp_job   = eligible ? tc.take<uint32_t>(hit_capacity) : nullptr;
-    int32_t*  dp_score = eligible ? tc.take<int32_t>(hit_capacity) : nullptr;
-    uint2*    dp_sink  = eligible ? tc.take<uint2>(hit_capacity) : nullptr;
-    uint32_t* dp_count = eligible ? tc.take<uint32_t>(4) : nullptr;
-    uint32_t* hit_string = per_read ? nullptr : tc.take<uint32_t>(hit_capacity);
-    uint32_t* p_off      = per_read ? nullptr : tc.take<uint32_t>(hit_capacity);
-    uint32_t* p_len      = per_read ? nullptr : tc.take<uint32_t>(hit_capacity);
-    uint32_t* t_off      = per_read ? nullptr : tc.take<uint32_t>(hit_capacity);
-    uint32_t* t_len      = per_read ? nullptr : tc.take<uint32_t>(hit_capacity);
-    int32_t*  h_score    = d_hit_score ? d_hit_score : (per_read ? nullptr : tc.take<int32_t>(hit_capacity));
-    uint2*    h_sink     = d_hit_sink ? (uint2*)d_hit_sink : (per_read ? nullptr : tc.take<uint2>(hit_capacity));
-    unsigned long long* best_key = tc.take<unsigned long long>(n_reads);
-    uint8_t* rb_strand = tc.take<uint8_t>((size_t)n_reads + 16);      // strand of every read's best alignment
-    size_t scan_bytes = 0, scan2_bytes = 0;
-    NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, sizes, excl, (int)nq, as_stream(stream)));
-    if (dedup && !per_read && hit_capacity) {
-        NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan2_bytes, flag, job_idx, (int)hit_capacity, as_stream(stream)));
-        if (scan2_bytes > scan_bytes) scan_bytes = scan2_bytes;
-    }
-    char* scan_tmp  = tc.take<char>(scan_bytes);
-    char* gotoh_tmp = tc.take<char>(gotoh_bytes);
-    // best-alignment traceback: per-read job arrays + the traceback's own temp (direction matrices)
-    uint32_t *bp_off = nullptr, *bp_len = nullptr, *bt_off = nullptr, *bt_len = nullptr; int32_t* b_score = nullptr;
-    uint2 *b_sink = nullptr, *b_source = nullptr; char* tb_tmp = nullptr; size_t tb_bytes = 0;
-    if (BA) {
-        bp_off = tc.take<uint32_t>(n_reads); bp_len = tc.take<uint32_t>(n_reads);
-        bt_off = tc.take<uint32_t>(n_reads); bt_len = tc.take<uint32_t>(n_reads);
-        b_score = tc.take<int32_t>(n_reads); b_sink = tc.take<uint2>(n_reads); b_source = tc.take<uint2>(n_reads);
-        const int r = nvb_banded_gotoh_traceback(P->band_len, P->type, &P->scheme, &pats, nullptr, &txts, n_reads,
-                                                 nullptr, nullptr, nullptr, nullptr, BA->max_ops, nullptr, nullptr, &tb_bytes, stream);
-        if (r != NVB_E_TEMP_SIZE && r != NVB_OK) return r;
-        tb_tmp = tc.take<char>(tb_bytes);
-    }
-    // paired-end stage: job slots (2 per pair), compacted full-DP jobs and the DP's own temp
-    uint32_t *pw_want = nullptr, *pw_idx = nullptr, *pw_pstr = nullptr, *pw_toff = nullptr, *pw_tlen = nullptr, *pcounts = nullptr;
-    uint32_t *rp_off = nullptr, *rp_len = nullptr, *rt_off = nullptr, *rt_len = nullptr; int32_t* rs_score = nullptr; uint2* rs_sink = nullptr;
-    char *pscan_tmp = nullptr, *full_tmp = nullptr; size_t pscan_bytes = 0, full_bytes = 0;
-    nvb_string_set rpats = pats, rtxts = txts;
-    if (PP) {
-        const uint32_t cap = PP->rescue_capacity;
-        pw_want = tc.take<uint32_t>(n_reads); pw_idx = tc.take<uint32_t>(n_reads); pw_pstr = tc.take<uint32_t>(n_reads);
-        pw_toff = tc.take<uint32_t>(n_reads); pw_tlen = tc.take<uint32_t>(n_reads); pcounts = tc.take<uint32_t>(4);
-        rp_off = tc.take<uint32_t>(cap); rp_len = tc.take<uint32_t>(cap); rt_off = tc.take<uint32_t>(cap); rt_len = tc.take<uint32_t>(cap);
-        rs_score = tc.take<int32_t>(cap); rs_sink = tc.take<uint2>(cap);
-        NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, pscan_bytes, pw_want, pw_idx, (int)n_reads, as_stream(stream)));
-        pscan_tmp = tc.take<char>(pscan_bytes);
-        rtxts.length = PP->max_frag;
-        const int r = nvb_gotoh_score_indirect(P->type, &P->scheme, &rpats, nullptr, &rtxts, (const uint32_t*)16, cap, (int32_t*)16, (nvb_uint2*)16,
-                                               nullptr, &full_bytes, stream);
-        if (r != NVB_E_TEMP_SIZE && r != NVB_OK) return r;
-        full_tmp = tc.take<char>(full_bytes);
-    }
+    p.eligible = p.per_read && shortcut_eligible(P->type, g.bits, P->band_len, P->scheme);
+    p.shortcut = p.eligible && g_perfect_shortcut.load(std::memory_order_relaxed);     // (the switch does not change the temp layout)
+    p.locate = p.per_read && c.f.sa_shift == 0u;
+    p.split = p.locate && c.f.ktab_k && g.seed_len > c.f.ktab_k && g_seed_split.load(std::memory_order_relaxed);
+    TempCarver tc(d_temp);
+    PIPE_TRY(carve_temp(c, tc, d_hit_score, d_hit_sink, BA, PP));
     const size_t need = tc.total();
     if (!d_temp || *temp_bytes < need) { *temp_bytes = need; return NVB_E_TEMP_SIZE; }
     if (n_reads == 0) return NVB_OK;
-
-    cudaStream_t s = as_stream(stream);
-    const FmIndex f = make_fmindex(fmi);
-    const StrSet rd = make_strset(reads);
     StageEvents* SE = nullptr;
-    { const int r = default_stage_events(&SE); if (r != NVB_OK) return r; }
-    NVB_STAGE(0);
-
-    // 1. [fw, rc] strings
-    {
-        const uint64_t total_words = (uint64_t)g.n_strings * (g.stride / spw);
-        const uint32_t grid = (uint32_t)((total_words + 255) / 256);
-        if (g.bits == 2 && rd.big_endian) pipe_make_strings_2bit_be_kernel<<<grid, 256, 0, s>>>(rd, g, str_words, str_len_);
-        else if (g.bits == 2)             pipe_make_strings_kernel<2><<<grid, 256, 0, s>>>(rd, g, str_words, str_len_);
-        else                              pipe_make_strings_kernel<4><<<grid, 256, 0, s>>>(rd, g, str_words, str_len_);
-        NVB_LAUNCH_CHECK();
-        if (str_quals) {
-            const uint64_t total = (uint64_t)g.n_strings * g.stride;
-            pipe_make_quals_kernel<<<(uint32_t)((total + 255) / 256), 256, 0, s>>>(rd, g, P->d_read_quals, str_quals);
-            NVB_LAUNCH_CHECK();
-        }
-    }
-    NVB_STAGE(1);
-    // 2. seed ranges
-    {
-        const uint32_t grid = (nq + SEED_BLOCK - 1) / SEED_BLOCK;
-        // per-read path + full suffix array: single-row ranges are located inside the match kernel (g_pipe_path 2 switches that off)
-        const uint32_t* loc_genome = (per_read && f.sa_shift == 0u && g_pipe_path != 2) ? d_genome : nullptr;
-        // with a k-mer table the located path runs in two passes: seeds on k-mers with >= 3 occurrences are finished by a second kernel
-        // (the lists live in `excl`, which the scan below overwrites)
-        const bool split = loc_genome && f.ktab_k && g.seed_len > f.ktab_k && g_seed_split;
-        if (split) {
-            NVB_CUDA_TRY(cudaMemsetAsync(seed_todo_n, 0, SEED_TODO_LISTS * SEED_TODO_PITCH * sizeof(uint32_t), s));
-            const uint32_t grid1 = (grid + SEED_ITER - 1u) / SEED_ITER;
-            if (g.bits == 2) pipe_seed_match_kernel<2, true><<<grid1, SEED_BLOCK, 0, s>>>(f, g, str_words, str_len_, loc_genome, ranges, sizes, excl, seed_todo_n);
-            else             pipe_seed_match_kernel<4, true><<<grid1, SEED_BLOCK, 0, s>>>(f, g, str_words, str_len_, loc_genome, ranges, sizes, excl, seed_todo_n);
-            NVB_LAUNCH_CHECK();
-            const uint32_t wgrid = SEED_TODO_LISTS * 37u;                                  // 2368 CTAs = 148 SMs x 16 resident CTAs
-            if (g.bits == 2) pipe_seed_match_wide_kernel<2><<<wgrid, SEED_BLOCK, 0, s>>>(f, g, str_words, loc_genome, ranges, sizes, excl, seed_todo_n, grid1);
-            else             pipe_seed_match_wide_kernel<4><<<wgrid, SEED_BLOCK, 0, s>>>(f, g, str_words, loc_genome, ranges, sizes, excl, seed_todo_n, grid1);
-        } else {
-            if (g.bits == 2) pipe_seed_match_kernel<2, false><<<grid, SEED_BLOCK, 0, s>>>(f, g, str_words, str_len_, loc_genome, ranges, sizes, nullptr, nullptr);
-            else             pipe_seed_match_kernel<4, false><<<grid, SEED_BLOCK, 0, s>>>(f, g, str_words, str_len_, loc_genome, ranges, sizes, nullptr, nullptr);
-        }
-        NVB_LAUNCH_CHECK();
-    }
-    NVB_STAGE(2);
-    // 3. hit slots
-    NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, sizes, excl, (int)nq, s));
-    pipe_count_kernel<<<1, 32, 0, s>>>(excl, sizes, nq, hit_capacity, counts);
-    NVB_LAUNCH_CHECK();
+    if (record_stages) PIPE_TRY(default_stage_events(&SE));
+    c.ev = SE ? SE->ev : nullptr;
+    NVB_STAGE(0); PIPE_TRY(run_strings(c));
+    NVB_STAGE(1); PIPE_TRY(run_seed_match(c));
+    NVB_STAGE(2); PIPE_TRY(run_hit_slots(c));
     NVB_STAGE(3);
-    // 4. locate + windows
-    const uint32_t hgrid = (hit_capacity + 255) / 256;
-    if (per_read) {
-        // 4'. per read: locate, window, distinct jobs; 5'. extension; 6'. best job per read
-        NVB_CUDA_TRY(cudaMemsetAsync(counts + 2, 0, sizeof(uint32_t), s));
-        NVB_CUDA_TRY(cudaMemsetAsync(best_key, 0, sizeof(unsigned long long) * n_reads, s));
-        if (hit_capacity) {
-            pipe_read_jobs_kernel<<<(n_reads + RJ_BLOCK - 1) / RJ_BLOCK, RJ_BLOCK, 0, s>>>(f, g, ranges, sizes, excl, str_len_, counts,
-                                                                                          j_string, j_first, jp_off, jp_len, jt_off, jt_len);
-            NVB_LAUNCH_CHECK();
-        }
-        NVB_STAGE(4);
-        NVB_STAGE(5);
-        if (hit_capacity && shortcut) {
-            const uint32_t jgrid = hgrid < 148u * 8u ? hgrid : 148u * 8u;
-            NVB_CUDA_TRY(cudaMemsetAsync(dp_count, 0, sizeof(uint32_t), s));
-            pipe_perfect_jobs_kernel<<<jgrid, 256, 0, s>>>(g, SC.match, SC.mismatch, SC.pattern_gap_open > SC.text_gap_open ? SC.pattern_gap_open : SC.text_gap_open, counts, str_words, d_genome, jp_off, jp_len, jt_off, jt_len, job_score, job_sink,
-                                                           dp_p_off, dp_p_len, dp_t_off, dp_t_len, dp_job, dp_count);
-            NVB_LAUNCH_CHECK();
-            size_t gb = gotoh_bytes;
-            pats.d_words = str_words; pats.d_offsets = dp_p_off; pats.d_lengths = dp_p_len;
-            txts.d_words = d_genome;  txts.d_offsets = dp_t_off; txts.d_lengths = dp_t_len;
-            const int r = nvb_banded_gotoh_score_indirect(P->band_len, P->type, &P->scheme, &pats, str_quals, &txts, dp_count, hit_capacity,
-                                                          dp_score, (nvb_uint2*)dp_sink, gotoh_tmp, &gb, stream);
-            if (r != NVB_OK) return r;
-            pipe_scatter_dp_kernel<<<jgrid, 256, 0, s>>>(dp_count, dp_job, dp_score, dp_sink, job_score, job_sink);
-            NVB_LAUNCH_CHECK();
-        } else if (hit_capacity) {
-            size_t gb = gotoh_bytes;
-            pats.d_words = str_words; pats.d_offsets = jp_off; pats.d_lengths = jp_len;
-            txts.d_words = d_genome;  txts.d_offsets = jt_off; txts.d_lengths = jt_len;
-            const int r = nvb_banded_gotoh_score_indirect(P->band_len, P->type, &P->scheme, &pats, str_quals, &txts, counts + 2, hit_capacity,
-                                                          job_score, (nvb_uint2*)job_sink, gotoh_tmp, &gb, stream);
-            if (r != NVB_OK) return r;
-        }
-        NVB_STAGE(6);
-        pipe_init_best_kernel<<<(n_reads + 255) / 256, 256, 0, s>>>(n_reads, d_best_score, d_best_pos, rb_strand);
-        NVB_LAUNCH_CHECK();
-        if (hit_capacity) {
-            // the job count lives on the device: a resident grid striding over it instead of hit_capacity / 256 mostly empty CTAs
-            const uint32_t jgrid = hgrid < 148u * 16u ? hgrid : 148u * 16u;
-            pipe_reduce_jobs_kernel<<<jgrid, 256, 0, s>>>(g, counts, j_string, j_first, job_score, best_key);
-            NVB_LAUNCH_CHECK();
-            pipe_finalize_jobs_kernel<<<jgrid, 256, 0, s>>>(g, counts, j_string, j_first, jt_off, job_score, job_sink, best_key,
-                                                            d_best_score, d_best_pos, rb_strand);
-            NVB_LAUNCH_CHECK();
-        }
-    } else {
-    if (hit_capacity) {
-        pipe_expand_hits_kernel<<<(nq + 255) / 256, 256, 0, s>>>(f, g, ranges, sizes, excl, str_len_, counts, hit_string, p_off, p_len, t_off, t_len);
-        NVB_LAUNCH_CHECK();
-    }
-    NVB_STAGE(4);
-    // 4b. collapse identical (string, window) jobs
-    if (dedup && hit_capacity) {
-        pipe_find_leaders_kernel<<<hgrid, 256, 0, s>>>(counts, hit_string, t_off, t_len, leader, flag);
-        NVB_LAUNCH_CHECK();
-        // the scan runs over the whole capacity; job_idx[h] depends only on flag[0..h), so the (unwritten) entries
-        // past counts[0] cannot influence any index that is read back
-        size_t sb = scan_bytes;
-        NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(scan_tmp, sb, flag, job_idx, (int)hit_capacity, s));
-        pipe_job_count_kernel<<<1, 32, 0, s>>>(job_idx, flag, counts);
-        NVB_LAUNCH_CHECK();
-        pipe_compact_jobs_kernel<<<hgrid, 256, 0, s>>>(counts, flag, job_idx, p_off, p_len, t_off, t_len, jp_off, jp_len, jt_off, jt_len);
-        NVB_LAUNCH_CHECK();
-    }
-    NVB_STAGE(5);
-    NVB_CUDA_TRY(cudaMemsetAsync(best_key, 0, sizeof(unsigned long long) * n_reads, s));
-    // 5. extension
-    if (hit_capacity) {
-        size_t gb = gotoh_bytes;
-        int r;
-        if (dedup) {
-            pats.d_words = str_words; pats.d_offsets = jp_off; pats.d_lengths = jp_len;
-            txts.d_words = d_genome;  txts.d_offsets = jt_off; txts.d_lengths = jt_len;
-            r = nvb_banded_gotoh_score_indirect(P->band_len, P->type, &P->scheme, &pats, str_quals, &txts, counts + 2, hit_capacity,
-                                                job_score, (nvb_uint2*)job_sink, gotoh_tmp, &gb, stream);
-            if (r != NVB_OK) return r;
-            pipe_scatter_scores_kernel<<<hgrid, 256, 0, s>>>(g, counts, leader, job_idx, job_score, job_sink, hit_string, h_score, h_sink, best_key);
-            NVB_LAUNCH_CHECK();
-        } else {
-            pats.d_words = str_words; pats.d_offsets = p_off; pats.d_lengths = p_len;
-            txts.d_words = d_genome;  txts.d_offsets = t_off; txts.d_lengths = t_len;
-            r = nvb_banded_gotoh_score_indirect(P->band_len, P->type, &P->scheme, &pats, str_quals, &txts, counts, hit_capacity,
-                                                h_score, (nvb_uint2*)h_sink, gotoh_tmp, &gb, stream);
-            if (r != NVB_OK) return r;
-        }
-    }
-    NVB_STAGE(6);
-    // 6. best per read (with job de-duplication the reduction already happened in the scatter kernel)
-    if (hit_capacity && !dedup) {
-        pipe_reduce_kernel<<<hgrid, 256, 0, s>>>(g, counts, hit_string, h_score, best_key);
-        NVB_LAUNCH_CHECK();
-    }
-    pipe_finalize_kernel<<<(n_reads + 255) / 256, 256, 0, s>>>(g, best_key, t_off, h_sink, hit_string, d_best_score, d_best_pos, rb_strand);
-    NVB_LAUNCH_CHECK();
-    }
-    if (hit_capacity && (d_hit_read || d_hit_window)) {
-        pipe_export_hits_kernel<<<hgrid, 256, 0, s>>>(g, counts, hit_string, t_off, t_len, d_hit_read, (uint2*)d_hit_window);
-        NVB_LAUNCH_CHECK();
-    }
-    if (BA) {
-        const uint32_t rgrid = (n_reads + 255) / 256;
-        pipe_best_jobs_kernel<<<rgrid, 256, 0, s>>>(g, best_key, hit_string, p_off, p_len, t_off, t_len, bp_off, bp_len, bt_off, bt_len, BA->d_strand);
-        NVB_LAUNCH_CHECK();
-        pats.d_words = str_words; pats.d_offsets = bp_off; pats.d_lengths = bp_len;
-        txts.d_words = d_genome;  txts.d_offsets = bt_off; txts.d_lengths = bt_len;
-        size_t tbb = tb_bytes;
-        const int r = nvb_banded_gotoh_traceback(P->band_len, P->type, &P->scheme, &pats, str_quals, &txts, n_reads,
-                                                 b_score, (nvb_uint2*)b_sink, (nvb_uint2*)b_source, BA->d_ops, BA->max_ops, BA->d_n_ops,
-                                                 tb_tmp, &tbb, stream);
-        if (r != NVB_OK) return r;
-        pipe_best_begin_kernel<<<rgrid, 256, 0, s>>>(g, best_key, bt_off, b_source, BA->d_n_ops, (uint2*)BA->d_begin);
-        NVB_LAUNCH_CHECK();
-    }
-    if (PP) {
-        const uint32_t n_pairs = n_reads / 2u, cap = PP->rescue_capacity;
-        const uint32_t pgrid = (n_pairs + 255) / 256, sgrid = (n_reads + 255) / 256;
-        pair_classify_kernel<<<pgrid, 256, 0, s>>>(g, n_pairs, *PP, d_best_score, d_best_pos, rb_strand, str_len_,
-                                                    pw_want, pw_pstr, pw_toff, pw_tlen, PO->d_pair_score, PO->d_pair_flags,
-                                                    PO->d_mate_score, PO->d_mate_pos, PO->d_mate_strand);
-        NVB_LAUNCH_CHECK();
-        size_t sb = pscan_bytes;
-        NVB_CUDA_TRY(cub::DeviceScan::ExclusiveSum(pscan_tmp, sb, pw_want, pw_idx, (int)n_reads, s));
-        pair_job_count_kernel<<<1, 32, 0, s>>>(pw_idx, pw_want, n_reads, cap, pcounts);
-        NVB_LAUNCH_CHECK();
-        if (cap) {
-            pair_compact_kernel<<<sgrid, 256, 0, s>>>(g, n_reads, cap, pw_want, pw_idx, pw_pstr, pw_toff, pw_tlen, str_len_, rp_off, rp_len, rt_off, rt_len);
-            NVB_LAUNCH_CHECK();
-            rpats.d_words = str_words; rpats.d_offsets = rp_off; rpats.d_lengths = rp_len;
-            rtxts.d_words = d_genome;  rtxts.d_offsets = rt_off; rtxts.d_lengths = rt_len;
-            size_t fb = full_bytes;
-            const int r = nvb_gotoh_score_indirect(P->type, &P->scheme, &rpats, str_quals, &rtxts, pcounts, cap, rs_score, (nvb_uint2*)rs_sink, full_tmp, &fb, stream);
-            if (r != NVB_OK) return r;
-        }
-        pair_finalize_kernel<<<pgrid, 256, 0, s>>>(n_pairs, *PP, pw_want, pw_idx, pw_toff, rs_score, rs_sink, PO->d_pair_score, PO->d_pair_flags,
-                                                    PO->d_mate_score, PO->d_mate_pos, PO->d_mate_strand);
-        NVB_LAUNCH_CHECK();
-        if (PO->d_n_rescue) NVB_CUDA_TRY(cudaMemcpyAsync(PO->d_n_rescue, pcounts, 2 * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
-    }
-    if (!dedup) NVB_CUDA_TRY(cudaMemcpyAsync(counts + 2, counts, sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
-    if (d_n_hits) NVB_CUDA_TRY(cudaMemcpyAsync(d_n_hits, counts, 3 * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
+    if (c.plan.per_read) PIPE_TRY(run_per_read(c, d_best_score, d_best_pos));
+    else                 PIPE_TRY(run_per_hit(c, d_best_score, d_best_pos, d_hit_read, d_hit_window));
+    if (BA) PIPE_TRY(run_traceback(c, BA));
+    if (PP) PIPE_TRY(run_paired(c, PP, PO, d_best_score, d_best_pos));
+    if (!c.plan.dedup) NVB_CUDA_TRY(cudaMemcpyAsync(c.t.counts + 2, c.t.counts, sizeof(uint32_t), cudaMemcpyDeviceToDevice, c.s));
+    if (d_n_hits) NVB_CUDA_TRY(cudaMemcpyAsync(d_n_hits, c.t.counts, 3 * sizeof(uint32_t), cudaMemcpyDeviceToDevice, c.s));
     NVB_STAGE(7);
-    SE->valid = true;
+    if (SE) SE->valid.store(true, std::memory_order_release);
     return NVB_OK;
 }
 
-extern "C" void nvb_debug_pipeline_path(int path) { g_pipe_path = path; }
-extern "C" void nvb_debug_seed_split(int on) { g_seed_split = on; }
-extern "C" void nvb_debug_perfect_shortcut(int on) { g_perfect_shortcut = on; }
-
-extern "C" int nvb_seed_extend(const nvb_fm_index* fmi, const uint32_t* d_genome,
-                    const nvb_string_set* reads, uint32_t n_reads,
-                    const nvb_seed_extend_params* P, uint32_t hit_capacity,
-                    int32_t* d_best_score, uint32_t* d_best_pos,
-                    uint32_t* d_n_hits, uint32_t* d_hit_read, nvb_uint2* d_hit_window,
-                    int32_t* d_hit_score, nvb_uint2* d_hit_sink,
+extern "C" int nvb_seed_extend(const nvb_fm_index* fmi, const uint32_t* d_genome, const nvb_string_set* reads, uint32_t n_reads,
+                    const nvb_seed_extend_params* P, uint32_t hit_capacity, int32_t* d_best_score, uint32_t* d_best_pos,
+                    uint32_t* d_n_hits, uint32_t* d_hit_read, nvb_uint2* d_hit_window, int32_t* d_hit_score, nvb_uint2* d_hit_sink,
                     void* d_temp, size_t* temp_bytes, void* stream)
 {
     return seed_extend_impl(fmi, d_genome, reads, n_reads, P, hit_capacity, d_best_score, d_best_pos, d_n_hits, d_hit_read, d_hit_window,
-                            d_hit_score, d_hit_sink, nullptr, nullptr, nullptr, d_temp, temp_bytes, stream);
+                            d_hit_score, d_hit_sink, nullptr, nullptr, nullptr, d_temp, temp_bytes, stream, true);
 }
 
-extern "C" int nvb_seed_extend_traceback(const nvb_fm_index* fmi, const uint32_t* d_genome,
-                    const nvb_string_set* reads, uint32_t n_reads,
-                    const nvb_seed_extend_params* P, uint32_t hit_capacity,
-                    int32_t* d_best_score, uint32_t* d_best_pos,
-                    uint32_t* d_n_hits, uint32_t* d_hit_read, nvb_uint2* d_hit_window,
-                    int32_t* d_hit_score, nvb_uint2* d_hit_sink,
-                    const nvb_best_alignment_out* best_alignment,
-                    void* d_temp, size_t* temp_bytes, void* stream)
+extern "C" int nvb_seed_extend_traceback(const nvb_fm_index* fmi, const uint32_t* d_genome, const nvb_string_set* reads, uint32_t n_reads,
+                    const nvb_seed_extend_params* P, uint32_t hit_capacity, int32_t* d_best_score, uint32_t* d_best_pos,
+                    uint32_t* d_n_hits, uint32_t* d_hit_read, nvb_uint2* d_hit_window, int32_t* d_hit_score, nvb_uint2* d_hit_sink,
+                    const nvb_best_alignment_out* best_alignment, void* d_temp, size_t* temp_bytes, void* stream)
 {
     if (!best_alignment) return NVB_E_INVALID;
     return seed_extend_impl(fmi, d_genome, reads, n_reads, P, hit_capacity, d_best_score, d_best_pos, d_n_hits, d_hit_read, d_hit_window,
-                            d_hit_score, d_hit_sink, best_alignment, nullptr, nullptr, d_temp, temp_bytes, stream);
+                            d_hit_score, d_hit_sink, best_alignment, nullptr, nullptr, d_temp, temp_bytes, stream, true);
 }
 
-extern "C" int nvb_seed_extend_paired(const nvb_fm_index* fmi, const uint32_t* d_genome,
-                    const nvb_string_set* reads, uint32_t n_pairs,
-                    const nvb_seed_extend_params* P, uint32_t hit_capacity,
-                    const nvb_pair_params* pair_params, const nvb_pair_out* out,
+extern "C" int nvb_seed_extend_paired(const nvb_fm_index* fmi, const uint32_t* d_genome, const nvb_string_set* reads, uint32_t n_pairs,
+                    const nvb_seed_extend_params* P, uint32_t hit_capacity, const nvb_pair_params* pair_params, const nvb_pair_out* out,
                     uint32_t* d_n_hits, void* d_temp, size_t* temp_bytes, void* stream)
 {
     if (!pair_params || !out || n_pairs > 0x3FFFFFFFu || !temp_bytes) return NVB_E_INVALID;
     // the per-read best (score, end) of the single-end stage lands in the mate arrays first and is then refined per pair
     return seed_extend_impl(fmi, d_genome, reads, 2u * n_pairs, P, hit_capacity, out->d_mate_score, out->d_mate_pos, d_n_hits, nullptr, nullptr,
-                            nullptr, nullptr, nullptr, pair_params, out, d_temp, temp_bytes, stream);
+                            nullptr, nullptr, nullptr, pair_params, out, d_temp, temp_bytes, stream, true);
 }

@@ -139,6 +139,23 @@ void hh_gapless_job_shortcut(const uint32_t* str_words, const uint32_t* genome_w
     }
 }
 
+// the per-hit rules of the seed + extend composition over n inputs
+void hh_hit_window(const uint32_t* pos, const uint32_t* seed_begin, const uint32_t* len, const uint32_t* band, const uint32_t* genome_len,
+                   uint32_t n, uint32_t* window) {
+    for (uint32_t a = 0; a < n; ++a) {
+        const uint2 w = hit_window(pos[a], seed_begin[a], len[a], band[a], genome_len[a]);
+        window[2 * a] = w.x; window[2 * a + 1] = w.y;
+    }
+}
+void hh_best_key(const int32_t* score, const uint32_t* hit, uint32_t n, unsigned long long* key, int32_t* key_score, uint32_t* key_hit) {
+    for (uint32_t a = 0; a < n; ++a) {
+        key[a] = best_key(score[a], hit[a]); key_score[a] = best_key_score(key[a]); key_hit[a] = best_key_hit(key[a]);
+    }
+}
+void hh_seed_range_size(const uint32_t* ranges, uint32_t n, uint32_t max_seed_hits, uint32_t* size) {
+    for (uint32_t a = 0; a < n; ++a) size[a] = seed_range_size(make_uint2(ranges[2 * a], ranges[2 * a + 1]), max_seed_hits);
+}
+
 // generic rank dictionary (dict_rank<W,I>): out[q] = rank(i[q], c[q]), all as uint64
 void hh_dict_rank(const void* text, uint32_t word_bits, const void* occ, uint32_t K, const uint64_t* qi, const uint8_t* qc, uint32_t nq, uint64_t* out) {
     for (uint32_t q = 0; q < nq; ++q) {

@@ -145,6 +145,28 @@ def test_unaligned_2bit_reads_and_streaming_api():
         assert torch.equal(nh, plain.n_hits.cpu())
 
 
+def test_stage_times_belong_to_the_last_direct_call(monkeypatch):
+    """last_stage_ms() reports the most recent direct seed_extend call: StreamingSeedExtend batches in flight on two compute streams
+    record no stage events and leave the reported times as they were"""
+    from nvbio_b200.pipeline import last_stage_ms
+    require_gpu()
+    n = 120_000
+    gw = synth.random_genome_words(n, seed=31)
+    fmi, _ = nb.FMIndexDevice.from_text(gw, n)
+    rw, _, _ = synth.sample_reads(gw, n, 1000, 150, seed=3, mut_seed=4)
+    nb.seed_extend(fmi, gw, PackedStringSet.fixed(rw.reshape(-1), 1000, 150, stride=rw.shape[1] * 16), nb.SeedExtendParams(), hit_capacity=64000)
+    before = last_stage_ms()
+    monkeypatch.setenv("NVB_PIPELINE_COMPUTE_STREAMS", "2")
+    st = nb.StreamingSeedExtend(fmi, gw, nb.SeedExtendParams(), 1000, 150, rw.shape[1], hit_capacity=64000, depth=2)
+    host = rw.cpu().pin_memory()
+    for _ in range(3):
+        for t in [st.submit(host) for _ in range(2)]:
+            st.result(t)
+    st.close()
+    torch.cuda.synchronize()
+    assert last_stage_ms() == before
+
+
 def test_best_alignment_traceback():
     """CIGAR of every read's best hit: re-applying the ops to the genome reproduces the read (up to its substitutions) and
     the score; equals the oracle traceback of the same (strand, window) job"""

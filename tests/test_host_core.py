@@ -798,12 +798,13 @@ def test_gotoh_window_quality_table(H, O):
                 ok = whole[3].astype(bool)
                 assert np.array_equal(sh["score"][ok], whole[0][ok]) and np.array_equal(sh["sx"][ok], whole[1][ok])
 
-@pytest.mark.parametrize("band", [31, 15, 8])
+@pytest.mark.parametrize("band", [31, 15, 8, 63])
 def test_gapless_job_shortcut(H, O, band, request):
     """gapless_job_shortcut (the exact shortcut of the LOCAL extension in nvb_seed_extend): whenever it claims a job, (score, sink) are
     exactly what the oracle's banded DP and the reference's own aln::banded_alignment_score<BAND> (oracle/_ref, bands 31 and 15) return -- reads with 0..4 substitutions at random and at chosen
     places (the ends, next to the ends, adjacent), reads with an indel (never provable), tandem repeats of period 1, 2, 3, 7 and 40 (other
-    band diagonals as good as the seed's), short and ragged reads, windows longer than the band needs, four schemes"""
+    band diagonals as good as the seed's), short and ragged reads, windows longer than the band needs, four schemes.  Jobs outside the
+    routine's preconditions are never claimed: band 63, and reads whose offset in their stream is not a multiple of 16"""
     rng = np.random.default_rng(900 + band)
     n_txt = 60_000
     text = rng.integers(0, 4, n_txt).astype(np.uint8)
@@ -836,23 +837,84 @@ def test_gapless_job_shortcut(H, O, band, request):
     po = (np.arange(n) * stride).astype(np.uint32)
     sw = np.concatenate([pack_symbols(reads.reshape(-1), 2, True), np.zeros(2, np.uint32)])
     gw = np.concatenate([pack_symbols(np.concatenate([text, np.zeros(64, np.uint8)]), 2, True), np.zeros(2, np.uint32)])
+    sw5 = np.concatenate([pack_symbols(np.concatenate([np.zeros(5, np.uint8), reads.reshape(-1)]), 2, True), np.zeros(2, np.uint32)])
+    po5 = po + np.uint32(5)                                             # the same reads 5 symbols further into their stream
     R = Reference(request, orc.Ref)
     total = 0
     for scheme in ((2, -2, -5, -3), (1, -4, -6, -1), (2, -6, -8, -3), (3, -1, -2, -2)):
+        solved = np.zeros(n, np.uint8); score = np.zeros(n, np.int32); sink = np.zeros((n, 2), np.uint32)
+        H.hh_gapless_job_shortcut(_p(sw5), _p(gw), _p(po5), _p(M), _p(to), _p(N), C.c_uint32(n), C.c_uint32(band), C.c_int32(scheme[0]), C.c_int32(scheme[1]),
+                                  C.c_int32(scheme[2]), _p(solved), _p(score), _p(sink))
+        assert not solved.any(), (band, scheme)
+        H.hh_gapless_job_shortcut(_p(sw), _p(gw), _p(po), _p(M), _p(to), _p(N), C.c_uint32(n), C.c_uint32(band), C.c_int32(scheme[0]), C.c_int32(scheme[1]),
+                                  C.c_int32(scheme[2]), _p(solved), _p(score), _p(sink))
+        ok = solved.astype(bool)
+        if band > 32:
+            assert not ok.any(), (band, scheme)
+            continue
         ws, wx, wy, _ = O.banded_gotoh(band, 1, scheme, reads.reshape(-1), po, M, text, to, N)
         if band in (31, 15):
             # ... and the reference's own aln::banded_alignment_score<BAND> (oracle/_ref) says the same as the restatement
             full = N >= M + band - 1                                    # (shorter windows: the reference reads past the text, undefined)
             R.same([ws[full], wx[full], wy[full]],
                    lambda: [r[full] for r in R.live.banded_gotoh(band, 1, scheme, reads.reshape(-1), po, M, text, to, N)[:3]])
-        solved = np.zeros(n, np.uint8); score = np.zeros(n, np.int32); sink = np.zeros((n, 2), np.uint32)
-        H.hh_gapless_job_shortcut(_p(sw), _p(gw), _p(po), _p(M), _p(to), _p(N), C.c_uint32(n), C.c_uint32(band), C.c_int32(scheme[0]), C.c_int32(scheme[1]),
-                                  C.c_int32(scheme[2]), _p(solved), _p(score), _p(sink))
-        ok = solved.astype(bool)
         assert np.array_equal(score[ok], ws[ok]) and np.array_equal(sink[ok, 0], wx[ok]) and np.array_equal(sink[ok, 1], wy[ok]), (band, scheme)
         assert not ok[N < M + band - 1].any()
         exact = (np.arange(n) % 7 == 0) | (np.arange(n) % 7 == 6)
         assert ok[exact & (N >= M + band - 1)].all()                     # a read without a difference is always resolved
         total += int(ok.sum())
         print("gapless_job_shortcut band %d scheme %s: %d of %d jobs claimed" % (band, scheme, int(ok.sum()), n))
-    assert total > 4 * n // 4
+    assert band > 32 or total > 4 * n // 4
+
+
+def test_hit_window(H):
+    """hit_window (the genome window of a hit on both extension paths) == the window rule of tests/pipeline_oracle.py clamped to the
+    text: seeds nearer the text start than their read offset, diagonals within band/2 of the text start, windows running past the
+    text's end, and the largest uint32 positions"""
+    rng = np.random.default_rng(41)
+    n = 3000
+    glen = rng.integers(1, 2**32, n, dtype=np.uint64)
+    pos = (rng.random(n) * glen).astype(np.uint64)
+    sb = rng.integers(0, 300, n, dtype=np.uint64); ln = rng.integers(1, 300, n, dtype=np.uint64); band = rng.integers(2, 64, n, dtype=np.uint64)
+    pos[:500] = sb[:500] // 2                                           # seed nearer the text start than its read offset
+    pos[500:1000] = sb[500:1000] + band[500:1000] // 2 - 1              # diagonal within band/2 of the text start
+    pos[1000:1500] = rng.integers(0, 10**6, 500, dtype=np.uint64); sb[1000:1500] = 0
+    glen[1000:1500] = pos[1000:1500] + 1 + ln[1000:1500] // 2           # window past the text's end
+    pos[1500:1600] = 0xFFFFFFFF; glen[1500:1600] = 0xFFFFFFFF           # the largest positions
+    ln[1550:1600] = 0xFFFFFFFF; band[1580:1600] = 0xFFFFFFFF
+    args = [u32(a) for a in (pos, sb, ln, band, glen)]
+    got = np.zeros((n, 2), np.uint32)
+    H.hh_hit_window(*[_p(a) for a in args], C.c_uint32(n), _p(got))
+    for a in range(n):
+        p, s, L, B, G = (int(v[a]) for v in (pos, sb, ln, band, glen))
+        diag = p - s if p > s else 0
+        gb = diag - B // 2 if diag > B // 2 else 0
+        assert (int(got[a, 0]), int(got[a, 1])) == (gb, min(gb + L + B, G)), (a, p, s, L, B, G)
+    assert (got[1000:1500, 1] == u32(glen[1000:1500])).all()
+
+
+def test_best_key(H):
+    """best_key orders the hits of a read as the best-per-read reduction needs: a higher score wins, an equal score goes to the smaller hit
+    index, negative scores sort below positive ones; score / hit <-> key round-trips and no hit packs to key 0 ("no hit")"""
+    rng = np.random.default_rng(43)
+    score = np.concatenate([[-2**31, -1, 0, 1, 2**31 - 1, -5, -5, 7, 7], rng.integers(-2**31, 2**31, 1000), rng.integers(-3, 4, 1000)]).astype(np.int32)
+    hit = np.concatenate([[0, 5, 5, 5, 0, 3, 4, 0, 0xFFFFFFFE], rng.integers(0, 0xFFFFFFFF, 1000), rng.integers(0, 20, 1000)]).astype(np.uint32)
+    n = len(score)
+    key = np.zeros(n, np.uint64); ks = np.zeros(n, np.int32); kh = np.zeros(n, np.uint32)
+    H.hh_best_key(_p(score), _p(hit), C.c_uint32(n), _p(key), _p(ks), _p(kh))
+    assert np.array_equal(ks, score) and np.array_equal(kh, hit) and (key != 0).all()
+    s, h = score.astype(np.int64), hit.astype(np.int64)
+    wins = (s[:, None] > s[None, :]) | ((s[:, None] == s[None, :]) & (h[:, None] < h[None, :]))
+    assert np.array_equal(key[:, None] > key[None, :], wins)
+    assert key[1] < key[3] and key[0] < key[2] and key[5] > key[6] and key[7] > key[8]
+
+
+def test_seed_range_size(H):
+    """seed_range_size (the hits a seed contributes, both extension paths and the seed match): an empty range contributes none, a range the
+    seed match already located (y = 0xFFFFFFFF) one, a row range its rows up to max_seed_hits"""
+    ranges = np.array([(1, 0), (9, 4), (0xFFFFFFFF, 0), (7, 7), (3, 12), (0, 0xFFFFFFFE), (123456, 0xFFFFFFFF), (0, 0xFFFFFFFF)], np.uint32)
+    for max_hits in (1, 5, 100, 0xFFFFFFFF):
+        got = np.zeros(len(ranges), np.uint32)
+        H.hh_seed_range_size(_p(np.ascontiguousarray(ranges)), C.c_uint32(len(ranges)), C.c_uint32(max_hits), _p(got))
+        want = [min(1 if y == 0xFFFFFFFF else (y - x + 1 if x <= y else 0), max_hits) for x, y in ranges.tolist()]
+        assert got.tolist() == want, max_hits

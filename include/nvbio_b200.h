@@ -391,7 +391,9 @@ typedef struct nvb_seed_extend_params {
 
 /* reads: n_reads strings (2- or 4-bit).  genome: 2-bit big-endian packed text of fmi->length symbols.
  * Outputs: d_best_score[n_reads] (INT_MIN when a read has no hit), d_best_pos[n_reads] = genome
- * coordinate of the best alignment's end (window begin + sink.x; 0xFFFFFFFF when none).
+ * coordinate of the best alignment's end (window begin + sink.x; 0xFFFFFFFF when none).  A read whose best job has a
+ * window shorter than the read (the read runs past the genome's end: no alignment fits) keeps the DP's score for it,
+ * -2^30, and gets d_best_pos 0xFFFFFFFF.
  * Optional per-hit outputs (may be NULL) of capacity hit_capacity: d_hit_read (string id = read*strands
  * + strand), d_hit_window (begin,end), d_hit_score, d_hit_sink; d_n_hits[0] receives the number of hits
  * kept (<= hit_capacity), d_n_hits[1] the number found and d_n_hits[2] the number of distinct alignment jobs
@@ -408,7 +410,9 @@ int nvb_seed_extend(const nvb_fm_index* fmi, const uint32_t* d_genome,
 /* Optional alignment of every read's best hit (what nvBowtie's banded_traceback_best produces for SAM output,
  * aligner_best_approx.h:300-500): the banded traceback of the best (strand, window) job of each read.
  *   d_ops[r*max_ops ..]  ops in END -> START order (0 M, 1 I, 2 D), d_n_ops[r] their number (0 when the read has no hit)
- *   d_begin[r]           = (genome coordinate of the alignment's first text symbol, first aligned read symbol)
+ *   d_begin[r]           = (genome coordinate of the alignment's first text symbol, first aligned read symbol);
+ *                          (0xFFFFFFFF, 0xFFFFFFFF) with n_ops 0 when the read has no hit, or when its best job's window is
+ *                          shorter than the read (no alignment: d_best_pos is 0xFFFFFFFF too)
  *   d_strand[r]          = 0 forward, 1 reverse complement (the read symbols are those of that strand's string)
  * Call with the same arguments as nvb_seed_extend plus this struct; temp size grows by the direction matrices. */
 typedef struct nvb_best_alignment_out {

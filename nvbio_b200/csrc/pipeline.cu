@@ -402,7 +402,7 @@ pipe_finalize_jobs_kernel(const PipeGeom g, const uint32_t* __restrict__ counts,
     for (uint32_t j = blockIdx.x * 256 + threadIdx.x; j < n; j += gridDim.x * 256) {
         const uint32_t s = j_string[j], read = s / g.strands;
         if (best_key[read] != nvb::best_key(job_score[j], j_first[j])) continue;
-        best_score[read] = job_score[j]; best_pos[read] = jt_off[j] + job_sink[j].x; best_strand[read] = (uint8_t)(s % g.strands);
+        best_score[read] = job_score[j]; best_pos[read] = hit_end(jt_off[j], job_sink[j].x); best_strand[read] = (uint8_t)(s % g.strands);
     }
 }
 
@@ -501,7 +501,7 @@ pipe_finalize_kernel(const PipeGeom g, const unsigned long long* __restrict__ be
     if (key == 0ull) { best_score[r] = INT_MIN; best_pos[r] = 0xFFFFFFFFu; if (best_strand) best_strand[r] = 0; return; }
     const uint32_t h = best_key_hit(key);
     best_score[r] = best_key_score(key);
-    best_pos[r] = t_off[h] + sink[h].x;
+    best_pos[r] = hit_end(t_off[h], sink[h].x);
     if (best_strand) best_strand[r] = (uint8_t)(hit_string[h] % g.strands);
 }
 
@@ -522,7 +522,8 @@ pipe_best_jobs_kernel(const PipeGeom g, const unsigned long long* __restrict__ b
     if (strand) strand[r] = (uint8_t)(hit_string[h] % g.strands);
 }
 
-// source cell (window-relative text start, read start) -> (genome coordinate, read start); reads without a hit: n_ops 0
+// source cell (window-relative text start, read start) -> (genome coordinate, read start); reads without a hit: n_ops 0.  A best job
+// without an alignment (window shorter than the read) has n_ops 0 and source (0xFFFFFFFF, 0xFFFFFFFF) from the traceback: see hit_end
 __global__ void __launch_bounds__(256)
 pipe_best_begin_kernel(const PipeGeom g, const unsigned long long* __restrict__ best_key, const uint32_t* __restrict__ bt_off,
                        const uint2* __restrict__ source, uint32_t* __restrict__ n_ops, uint2* __restrict__ begin)
@@ -531,7 +532,7 @@ pipe_best_begin_kernel(const PipeGeom g, const unsigned long long* __restrict__ 
     if (r >= g.n_reads) return;
     if (best_key[r] == 0ull) { n_ops[r] = 0; begin[r] = make_uint2(0xFFFFFFFFu, 0xFFFFFFFFu); return; }
     const uint2 sc = source[r];
-    begin[r] = make_uint2(bt_off[r] + sc.x, sc.y);
+    begin[r] = make_uint2(hit_end(bt_off[r], sc.x), sc.y);
 }
 
 __global__ void __launch_bounds__(256)

@@ -33,6 +33,14 @@ __host__ __device__ __forceinline__ uint2 hit_window(const uint32_t pos, const u
     return make_uint2(gb, ge < genome_len ? (uint32_t)ge : genome_len);
 }
 
+// Genome coordinate of an alignment's end (or, with a traceback's source cell, its begin): window begin + sink.x.  A job whose window is
+// shorter than its read (a read running past the genome's end) has no alignment: the DP leaves its sink at the default 0xFFFFFFFF (score
+// NVB_SINK_MIN), and the coordinate is 0xFFFFFFFF ("no position") instead of the wrapped sum window_begin - 1.
+__host__ __device__ __forceinline__ uint32_t hit_end(const uint32_t window_begin, const uint32_t sink_x)
+{
+    return sink_x == 0xFFFFFFFFu ? 0xFFFFFFFFu : window_begin + sink_x;
+}
+
 // Key of the best-per-read reduction (an atomicMax over the keys of a read's hits): the higher score wins, among equal scores the
 // smaller hit index.  The score's sign bit is flipped so that negative scores sort below positive ones; the hit index is stored as
 // 0xFFFFFFFF - hit.  Key 0 means "no hit": it would take score INT_MIN at hit 0xFFFFFFFF, beyond every hit capacity.

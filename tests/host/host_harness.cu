@@ -147,6 +147,9 @@ void hh_hit_window(const uint32_t* pos, const uint32_t* seed_begin, const uint32
         window[2 * a] = w.x; window[2 * a + 1] = w.y;
     }
 }
+void hh_hit_end(const uint32_t* window_begin, const uint32_t* sink_x, uint32_t n, uint32_t* end) {
+    for (uint32_t a = 0; a < n; ++a) end[a] = hit_end(window_begin[a], sink_x[a]);
+}
 void hh_best_key(const int32_t* score, const uint32_t* hit, uint32_t n, unsigned long long* key, int32_t* key_score, uint32_t* key_hit) {
     for (uint32_t a = 0; a < n; ++a) {
         key[a] = best_key(score[a], hit[a]); key_score[a] = best_key_score(key[a]); key_hit[a] = best_key_hit(key[a]);

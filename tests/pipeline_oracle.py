@@ -10,9 +10,19 @@ def _scheme_args(sch):
     return (sch.match, sch.mismatch, sch.gap_open, sch.gap_ext), None
 
 
-def seed_extend_oracle(O, idx, genome_sym, reads, params, quals=None):
+NO_POS = 0xFFFFFFFF
+
+
+def hit_end(window_begin, sink_x):
+    """genome coordinate window begin + sink.x of an alignment end (include/nvbio_b200.h, d_best_pos); NO_POS for the DP's default
+    sink 0xFFFFFFFF, which a window shorter than its read gets (no alignment fits)"""
+    return NO_POS if int(sink_x) == NO_POS else int(window_begin) + int(sink_x)
+
+
+def seed_extend_oracle(O, idx, genome_sym, reads, params, quals=None, hit_capacity=None):
     """reads: list of uint8 arrays; quals: optional list of uint8 arrays (base qualities, with a QualityGotohScheme).
-    Returns dict(best_score, best_pos, hit_string, hit_window, hit_score, hit_sink, n_hits)."""
+    hit_capacity: hits at index >= capacity are dropped (in hit order) and the best is taken over the kept hits only.
+    Returns dict(best_score, best_pos, best_hit (-1: none), hit_string, hit_window, hit_score, hit_sink, n_hits (kept), n_found)."""
     L, I, B = params.seed_len, params.seed_interval, params.band_len
     n = idx.n
     strands = 2 if params.both_strands else 1
@@ -40,44 +50,47 @@ def seed_extend_oracle(O, idx, genome_sym, reads, params, quals=None):
                 off.append(o); ln.append(0); valid.append(False)
     qcat = np.concatenate(q) if q else np.zeros(1, np.uint8)
     ranges, _ = O.match(idx, qcat, np.array(off, np.uint32), np.array(ln, np.uint32))
-    hit_string, rows, seed_k = [], [], []
-    for qi, ((x, y), v) in enumerate(zip(ranges, valid)):
-        if not v or x > y:
-            continue
-        sz = min(int(y) - int(x) + 1, params.max_seed_hits)
-        for j in range(sz):
-            hit_string.append(qi // K); seed_k.append(qi % K); rows.append(int(x) + j)
-    rows = np.array(rows, np.uint32)
-    pos = O.locate(idx, rows) if len(rows) else np.zeros(0, np.uint32)
-    p_sym, p_q, p_off, p_len, t_off, t_len, wins = [], [], [], [], [], [], []
-    po = 0
-    for s, k, p in zip(hit_string, seed_k, pos):
-        ln_s = len(strings[s])
-        sb = k * I
-        diag = int(p) - sb if int(p) > sb else 0
-        gb = diag - B // 2 if diag > B // 2 else 0
-        ge = min(gb + ln_s + B, n)
-        p_sym.append(strings[s]); p_off.append(po); p_len.append(ln_s); po += ln_s
-        if quals is not None:
-            p_q.append(squals[s])
-        t_off.append(gb); t_len.append(ge - gb); wins.append((gb, ge))
+    # hits in slot order: seed by seed (string, then seed), the first max_seed_hits rows of each range
+    x, y = ranges[:, 0].astype(np.int64), ranges[:, 1].astype(np.int64)
+    sz = np.where(np.array(valid, bool) & (x <= y), np.minimum(y - x + 1, params.max_seed_hits), 0)
+    n_found = int(sz.sum())
+    qi = np.repeat(np.arange(len(sz)), sz)
+    rows = (x[qi] + np.arange(n_found) - np.repeat(np.cumsum(sz) - sz, sz))
+    kept = n_found if hit_capacity is None else min(n_found, hit_capacity)
+    qi, rows = qi[:kept], rows[:kept]
+    hit_string, seed_begin = qi // K, (qi % K) * I
+    pos = O.locate(idx, rows.astype(np.uint32)).astype(np.int64) if kept else np.zeros(0, np.int64)
+    s_len = np.array([len(s) for s in strings], np.int64)
+    s_off = np.cumsum(s_len) - s_len
+    ln_s = s_len[hit_string]
+    diag = np.where(pos > seed_begin, pos - seed_begin, 0)
+    gb = np.where(diag > B // 2, diag - B // 2, 0)
+    ge = np.minimum(gb + ln_s + B, n)
+    wins = np.stack([gb, ge], axis=1)
     scheme, qtab = _scheme_args(params.scheme)
-    if hit_string:
-        score, sx, sy, _ = O.banded_gotoh(B, params.type, scheme, np.concatenate(p_sym), np.array(p_off, np.uint32), np.array(p_len, np.uint32),
-                                          genome_sym, np.array(t_off, np.uint32), np.array(t_len, np.uint32),
-                                          qual=np.concatenate(p_q) if quals is not None else None, qtab=qtab)
-    else:
-        score = np.zeros(0, np.int32); sx = sy = np.zeros(0, np.uint32)
+    score = np.zeros(kept, np.int64); sink = np.zeros((kept, 2), np.int64)
+    if kept:
+        # every distinct (string, window) job once; the patterns are the strings themselves
+        jobs, inv = np.unique(np.stack([hit_string, gb, ge], axis=1), axis=0, return_inverse=True)
+        inv = inv.reshape(-1)
+        sc, sx, sy, _ = O.banded_gotoh(B, params.type, scheme, np.concatenate(strings), s_off[jobs[:, 0]].astype(np.uint32),
+                                       s_len[jobs[:, 0]].astype(np.uint32), genome_sym, jobs[:, 1].astype(np.uint32),
+                                       (jobs[:, 2] - jobs[:, 1]).astype(np.uint32),
+                                       qual=np.concatenate(squals) if quals is not None else None, qtab=qtab)
+        score = sc.astype(np.int64)[inv]
+        sink = np.stack([sx.astype(np.int64), sy.astype(np.int64)], axis=1)[inv]
+    # best hit per read: max score, ties -> smallest hit index
     best_score = np.full(len(reads), -2**31, np.int64)
-    best_pos = np.full(len(reads), 0xFFFFFFFF, np.int64)
-    for h, s in enumerate(hit_string):
-        r = s // strands
-        if int(score[h]) > best_score[r]:
-            best_score[r] = int(score[h]); best_pos[r] = t_off[h] + int(sx[h])
-    return dict(best_score=best_score, best_pos=best_pos, hit_string=np.array(hit_string, np.int64),
-                hit_window=np.array(wins, np.int64).reshape(-1, 2), hit_score=score.astype(np.int64),
-                hit_sink=np.stack([sx.astype(np.int64), sy.astype(np.int64)], axis=1) if len(sx) else np.zeros((0, 2), np.int64),
-                n_hits=len(hit_string))
+    best_pos = np.full(len(reads), NO_POS, np.int64)
+    best_hit = np.full(len(reads), -1, np.int64)
+    read = hit_string // strands
+    order = np.lexsort((np.arange(kept), -score, read))
+    first = order[np.r_[True, read[order][1:] != read[order][:-1]]] if kept else order
+    for h in first.tolist():
+        r = int(read[h])
+        best_hit[r] = h; best_score[r] = int(score[h]); best_pos[r] = hit_end(gb[h], sink[h, 0])
+    return dict(best_score=best_score, best_pos=best_pos, best_hit=best_hit, hit_string=hit_string.astype(np.int64),
+                hit_window=wins.astype(np.int64).reshape(-1, 2), hit_score=score, hit_sink=sink.reshape(-1, 2), n_hits=kept, n_found=n_found)
 
 
 def seed_extend_paired_oracle(O, idx, genome_sym, reads, params, pair, n_pairs, quals=None):
@@ -88,21 +101,17 @@ def seed_extend_paired_oracle(O, idx, genome_sym, reads, params, pair, n_pairs, 
     se = seed_extend_oracle(O, idx, genome_sym, reads, params, quals=quals)
     glen = idx.n
     strands = 2
-    # best hit of every read: max score, ties -> smallest hit index
-    best_h = np.full(len(reads), -1, np.int64)
-    for h, s in enumerate(se["hit_string"]):
-        r = int(s) // strands
-        if best_h[r] < 0 or se["hit_score"][h] > se["hit_score"][best_h[r]]:
-            best_h[r] = h
+    best_h = se["best_hit"]
     INT_MIN = -2**31
 
     def mate(r):
+        # a mate is aligned when its best hit has a position (a window shorter than the read has none: hit_end)
         h = best_h[r]
-        if h < 0:
+        end = NO_POS if h < 0 else hit_end(se["hit_window"][h][0], se["hit_sink"][h][0])
+        if end == NO_POS:
             return dict(has=False, score=INT_MIN, strand=0, beg=0xFFFFFFFF, end=0xFFFFFFFF, len=0)
         s = int(se["hit_string"][h])
         ln = len(reads[r])
-        end = int(se["hit_window"][h][0] + se["hit_sink"][h][0])
         return dict(has=True, score=int(se["hit_score"][h]), strand=s % strands, beg=max(end - ln, 0), end=end, len=ln)
 
     cap = 2 * n_pairs if pair.rescue_capacity is None else pair.rescue_capacity

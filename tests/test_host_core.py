@@ -893,6 +893,21 @@ def test_hit_window(H):
     assert (got[1000:1500, 1] == u32(glen[1000:1500])).all()
 
 
+def test_hit_end(H):
+    """hit_end (a read's best_pos and its traceback's begin): window begin + sink.x for a sink the DP reported, 0xFFFFFFFF ("no position")
+    for the default sink of a window shorter than its read -- never the wrapped window_begin - 1 -- including windows that begin at 0"""
+    rng = np.random.default_rng(44)
+    wb = np.concatenate([[0, 0, 0, 1, 5, 199_885, 0xFFFFFFFE, 0xFFFFFFFF], rng.integers(0, 2**31, 500)]).astype(np.uint32)
+    sx = np.concatenate([[0, 7, 0xFFFFFFFF, 0xFFFFFFFF, 0xFFFFFFFF, 0xFFFFFFFF, 1, 0xFFFFFFFF], rng.integers(0, 400, 500)]).astype(np.uint32)
+    sx[100:200] = 0xFFFFFFFF
+    got = np.zeros(len(wb), np.uint32)
+    H.hh_hit_end(_p(wb), _p(sx), C.c_uint32(len(wb)), _p(got))
+    want = [0xFFFFFFFF if x == 0xFFFFFFFF else b + x for b, x in zip(wb.tolist(), sx.tolist())]
+    assert got.tolist() == want
+    assert got[:8].tolist() == [0, 7, 0xFFFFFFFF, 0xFFFFFFFF, 0xFFFFFFFF, 0xFFFFFFFF, 0xFFFFFFFF, 0xFFFFFFFF]
+    assert (got[100:200] == 0xFFFFFFFF).all() and (got[8:100] != 0xFFFFFFFF).all()
+
+
 def test_best_key(H):
     """best_key orders the hits of a read as the best-per-read reduction needs: a higher score wins, an equal score goes to the smaller hit
     index, negative scores sort below positive ones; score / hit <-> key round-trips and no hit packs to key 0 ("no hit")"""
